@@ -3,12 +3,15 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # the CUDA path
     python bench.py --impl reference [--gpus N] --steps K --warmup W  # the reference's CPU path
+    python bench.py --steps K --warmup W --dump-outputs DIR          # also write the last step's results
 
 A "step" = every chain runs successful neighbour proposals (mutate, repair, full cost, accept/undo)
-for `--step-ms` of SM clocks (a proposal cut by the deadline is suspended at a checkpoint and carried
-on by the next step, so every warp works to the end of the step), on the 1 MiB synthetic mixed
-text/binary input of BASELINE.json configs[1], all chains starting from the all-literal slab like
-the reference does (`--packet-budget` gives a reproducible budget instead).  `value` counts successful
+until it has priced `--packet-budget` packets (a proposal cut by the budget is suspended at a checkpoint
+and carried on by the next step), on the 1 MiB synthetic mixed text/binary input of BASELINE.json
+configs[1], all chains starting from the all-literal slab like the reference does.  The budget is work,
+not time, so the same arguments compute the same results on every run (see STEP_PACKETS for its cost).
+`--packet-budget 0` ends steps on `--step-ms` of SM clocks instead, which keeps every warp busy to the
+end of the step but makes how far the chains get depend on the clock.  `value` counts successful
 evaluations of ALL chains on ALL GPUs per second of device time (CUDA events on the library's
 launch stream, max over ranks).  `e2e` is the same metric through the one-shot host call with
 host buffers in and out (input upload, index build, chain allocation, best slab read-back).
@@ -39,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 from tools import corpus  # noqa: E402
 
@@ -46,6 +50,11 @@ METRIC = "neighbour_cost_evals_per_sec"
 UNIT = "evals/s"
 WORKLOAD = "1 MiB synthetic mixed text/binary (tools/corpus.py mixed, seed 7), all-literal start, reference schedule step 0"
 ISSUE_CEILING_BITS_PER_S = 148 * 1.965e9 * 32 / 3  # SURVEY.md §8(d): shared-memory bank ceiling for the scorer
+# packets each chain prices per step: the work a 1000 ms SM-clock step does from the all-literal start (5 timed steps
+# after 3 warm-up ones: 828 323 evaluations against 823 389), so that the timed steps see slabs of the same age.
+# Measured on a B200 at 1000 W and 1965 MHz: 1.26 s per step, 132 k evaluations/s against 164 k for --packet-budget 0,
+# because chains given equal work finish unevenly (warp busy fraction 0.79 against 1.00)
+STEP_PACKETS = 23_000_000
 
 
 def peaks():
@@ -238,7 +247,7 @@ def size_leg(mg, wave: int, budget_s: float, device: int) -> list:
     import lzma
     import tempfile
     from megalania_b200 import build
-    cli = build.build_cli() or build.CLI
+    cli = build.CLI  # as build() left it: the benchmark compiles nothing into the tree
     out = []
     for name, kind, n, chains in (("config 1: 64 KiB synthetic English-like text", "text", 65536, wave),
                                   ("config 2: 1 MiB synthetic mixed text/binary", "mixed", 1 << 20, wave),
@@ -322,6 +331,28 @@ def encode_leg(mg, data: bytes, best_slab, device: int) -> dict:
     return out
 
 
+DUMP_SEED, DUMP_CHAINS, DUMP_POSITIONS = 2024, 8, 65536
+
+
+def dump_outputs(an, out_dir: str, suffix: str = "") -> None:
+    """What the timed path leaves its caller after the last timed step, as DIR/<name><suffix>.npy: every chain's
+    current and best cost (float64, exact below 2^53) and, for a fixed seeded sample of chains and positions, the
+    (type, dist, len) of those slots of their current and best slabs (float32, exact: dist < 2^24).  About 12 MB
+    at the default size."""
+    os.makedirs(out_dir, exist_ok=True)
+    cur, best = an.costs()
+    rng = np.random.default_rng(DUMP_SEED)
+    chains = np.sort(rng.choice(an.chains, size=min(DUMP_CHAINS, an.chains), replace=False))
+    pos = np.sort(rng.choice(an.ctx.n, size=min(DUMP_POSITIONS, an.ctx.n), replace=False))
+    arrays = {"cur_cost": cur.astype(np.float64), "best_cost": best.astype(np.float64),
+              "sample_chains": chains.astype(np.float64), "sample_positions": pos.astype(np.float64)}
+    for name, is_best in (("cur_slab_sample", False), ("best_slab_sample", True)):
+        slots = np.stack([an.get_slab(int(c), best=is_best)[pos] for c in chains])
+        arrays[name] = np.stack([slots["type"], slots["dist"], slots["len"]], axis=-1).astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # the CUDA arm
 # ------------------------------------------------------------------------------------------------
@@ -343,7 +374,7 @@ def run_cuda(args) -> None:
         import torch.distributed as dist_mod
         dist = dist_mod
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    mg.load_library()
+    mg.load_library(build_if_missing=False)
     n = args.size
     data = _corpus("mixed", n)
     ctx = mg.Context(data, device=local)
@@ -351,8 +382,12 @@ def run_cuda(args) -> None:
     chains = args.chains or (props.multi_processor_count * args.warps_per_sm if args.warps_per_sm else ctx.full_wave())
     chain_bytes = ctx.chain_bytes(chains=chains, track_best=1)
     free, _ = torch.cuda.mem_get_info(local)
+    wanted = chains
     while chains > 8 and chains * chain_bytes > 0.85 * free:
         chains //= 2
+    if args.dump_outputs and chains != wanted:
+        raise SystemExit(f"bench.py: only {chains} of {wanted} chains fit in free device memory; a dump of the smaller "
+                         "population could not be compared with other runs")
     an = mg.Annealer(ctx, chains, seed=args.seed + 1000003 * rank)
     an.set_slab(None)
 
@@ -425,6 +460,8 @@ def run_cuda(args) -> None:
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     device_s = agg["kernel_ms"] / 1e3
+    if args.dump_outputs:
+        dump_outputs(an, args.dump_outputs, f"_rank{rank}" if world > 1 else "")
 
     # max over ranks (device time), sum over ranks (work)
     if dist is not None:
@@ -509,7 +546,8 @@ def run_cuda(args) -> None:
             dist.all_reduce(w, op=dist.ReduceOp.SUM)
             e2e_evals = int(w[0])
         e2e = {"value": e2e_evals / e2e_s, "unit": UNIT, "h2d_bytes_per_step": n, "d2h_bytes_per_step": 12 * n + 8,
-               "steps": args.e2e_steps, "step_ms": args.step_ms * args.e2e_step_factor,
+               "steps": args.e2e_steps, "step_ms": None if args.packet_budget else args.step_ms * args.e2e_step_factor,
+               "step_packets": args.packet_budget * args.e2e_step_factor or None,
                "call": "mg_ctx_create + mg_anneal_oneshot (host data in, best slab + cost out); every step uploads the input, "
                        "builds the index, allocates and fills the chains, anneals, reads the best slab back and frees everything"}
 
@@ -581,7 +619,7 @@ def run_cuda(args) -> None:
                           "finder_candidates": agg["finder_candidates"], "log_overflows": agg["log_overflows"],
                           "finder_share_of_warp_time": agg["finder_cycles"] / max(1, agg["chain_cycles"]),
                           "warp_busy_fraction": agg["chain_cycles"] / max(1, chains * agg["max_chain_cycles"]) * 1.0 if args.steps == 1 else None,
-                          "suspended_resumed": "proposals cut by the step deadline are finished by the next step"}}
+                          "suspended_resumed": "proposals cut at the end of a step are finished by the next step"}}
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if dist is not None:
@@ -599,9 +637,10 @@ def main() -> None:
     ap.add_argument("--chains", type=int, default=0, help="chains per GPU (default: SMs x --warps-per-sm)")
     ap.add_argument("--warps-per-sm", type=int, default=0, help="0 = the library's own figure (chains per SM that fit shared memory)")
     ap.add_argument("--evals", type=int, default=1_000_000, help="cap on successful evaluations per chain per step")
-    ap.add_argument("--step-ms", type=float, default=1000.0, help="length of a step in milliseconds of SM clocks")
-    ap.add_argument("--packet-budget", type=int, default=0,
-                    help="instead of --step-ms: a chain ends its step when it has priced this many packets (reproducible)")
+    ap.add_argument("--packet-budget", type=int, default=STEP_PACKETS,
+                    help="a chain ends its step when it has priced this many packets (reproducible); 0 = end steps on --step-ms")
+    ap.add_argument("--step-ms", type=float, default=1000.0,
+                    help="with --packet-budget 0: length of a step in milliseconds of SM clocks (results depend on the clock)")
     ap.add_argument("--seed", type=int, default=1673551)
     ap.add_argument("--exchange-every", type=int, default=4, help="multi-GPU: best-slab broadcast every this many steps")
     ap.add_argument("--t-min", type=float, default=16.0, help="multi-GPU: coldest ladder temperature, 1/2048 bit")
@@ -618,7 +657,14 @@ def main() -> None:
     ap.add_argument("--config3-seconds", type=float, default=4.0)
     ap.add_argument("--cpu-evals", type=int, default=0, help="evaluations of the CPU sample (default: sized to ~15 s)")
     ap.add_argument("--cpu-procs", type=int, default=1 << 30)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one left the chains with as DIR/<name>.npy "
+                         "(per-chain costs, a seeded sample of slab slots; _rank<r> suffixes under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the CUDA path's results")
     if args.cpu_evals == 0:
         # ~6.6 evals/s at 1 MiB on one core (BASELINE.md): ~15 s for the single-core sample,
         # ~2 s per step per core for the all-cores reference arm

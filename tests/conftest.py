@@ -19,15 +19,6 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference (oracle/_ref); skipped where it was never built."""
-    from oracle import oracle_lib
-    if not oracle_lib.ref_available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    return oracle_lib.Ref()
-
-
-@pytest.fixture(scope="session")
 def corpora():
     from tools import corpus
     cache = {}
