@@ -144,6 +144,25 @@ MG_API int mg_encode_slab_buffer(mg_ctx* ctx, const LZMAPacket* slab, uint8_t* o
  * by the last mg_encode_slab / mg_encode_slab_buffer on ctx. */
 MG_API int mg_encode_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* events);
 
+/* ---- stream -> slab: resume from an existing .lzma stream --------------------------------- */
+
+/* Replaces nothing in the reference (it has no way to read its output back).  Decodes an LZMA-alone stream of the
+ * context's input - an earlier megalania output, or e.g. liblzma's with lc = lp = pb = 0 - into the slab that encodes
+ * to it: the packet that starts at a position goes to that position's slot, every other slot is LITERAL / 0 / 1
+ * (packet_slab_new's value).  The range decoder runs on the device (one warp) with this project's model, the range
+ * coder of mg_encode_slab run backwards; the result can start a search anywhere a slab can (mg_anneal_set_slab,
+ * mg_anneal_oneshot).  stream: host, len bytes; out_slab: host, n packets.
+ *   MG_EINVAL: fewer than 13 + 5 bytes; a properties byte other than 0 (the message names the lc / lp / pb found);
+ *              a size field that is neither n nor all ones (unknown size).  The dictionary size is ignored.
+ *   MG_ESLAB:  the payload is not this input's: the range coder's first byte is not 0; a literal differs from the
+ *              input; a match or rep reaches before position 0, runs past n or copies bytes that differ; with the size
+ *              unknown, the end marker does not stand exactly at n; the stream ends early, has bytes left over, or the
+ *              decoder's code is not 0 at the end.  The message gives the position.  Every read is bounds-checked. */
+MG_API int mg_decode_stream(mg_ctx* ctx, const uint8_t* stream, size_t len, LZMAPacket* out_slab);
+/* Device time (CUDA events around the decoder kernel) and events decoded (modelled bits + direct-bit groups, the unit
+ * of mg_encode_stats) by the last mg_decode_stream on ctx. */
+MG_API int mg_decode_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* events);
+
 /* ---- the annealing loop ---------------------------------------------------------------- */
 
 enum {

@@ -5,6 +5,7 @@ The names follow the reference's vocabulary (slab, packet, top-k finder, perplex
   Context.score_slabs(slabs)    perplexity_encoder total of a slab          (src/perplexity_encoder.c)
   Context.find_topk(...)        top_k_packet_finder_find + pop loop         (src/top_k_packet_finder.c)
   Context.encode_slab(slab)     header + range_encoder pass                 (src/main.c:110-119)
+  Context.decode_stream(stream) .lzma stream (lc = lp = pb = 0) -> slab, to resume a search (no reference counterpart)
   Annealer(ctx, chains, ...)    the loop of src/main.c:78-102 on many chains
 
 There is no CPU path: importing works anywhere, but every compute call needs the CUDA library
@@ -87,6 +88,7 @@ EXPORTS = [
     "mg_comm_unique_id", "mg_comm_init", "mg_comm_destroy", "mg_comm_rank", "mg_comm_size", "mg_comm_exchange_best",
     "mg_comm_temper_exchange", "mg_temper_decide", "mg_comm_merge_regions", "mg_comm_stats", "mg_pool_trim",
     "mg_comm_broadcast_chain", "mg_comm_allgather_u64", "mg_ctx_set_finder_limits", "mg_anneal_greedy_init",
+    "mg_decode_stream", "mg_decode_stats",
 ]
 
 _lib = None
@@ -166,6 +168,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mg_comm_broadcast_chain.argtypes = [vp, i32, u32, u32]
     L.mg_comm_allgather_u64.argtypes = [vp, u64, vp]
     L.mg_encode_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
+    L.mg_decode_stream.argtypes = [vp, vp, sz, vp]
+    L.mg_decode_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
     _lib = L
     return L
 
@@ -286,6 +290,21 @@ class Context:
         _check(self._lib.mg_encode_slab_buffer(self._h, _slab_ptr(slab, self.n), out.ctypes.data_as(C.c_void_p), cap,
                                                C.byref(got)))
         return out[:got.value].tobytes()
+
+    def decode_stream(self, stream: bytes) -> np.ndarray:
+        """An LZMA-alone stream of this input (lc = lp = pb = 0: an earlier output, or liblzma's) -> the slab that
+        encodes to it, n packets; slots no packet starts at are LITERAL / 0 / 1.  Raises MegalaniaError with MG_EINVAL
+        (header) or MG_ESLAB (a payload that is not this input's)."""
+        buf = np.ascontiguousarray(np.frombuffer(bytes(stream), dtype=np.uint8))
+        out = np.zeros(self.n, dtype=PACKET_DTYPE)
+        _check(self._lib.mg_decode_stream(self._h, buf.ctypes.data_as(C.c_void_p), buf.size,
+                                          out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def decode_stats(self) -> dict:
+        ms, ev = C.c_double(0), C.c_uint64(0)
+        _check(self._lib.mg_decode_stats(self._h, C.byref(ms), C.byref(ev)))
+        return {"kernel_ms": ms.value, "events": int(ev.value)}
 
     def model_after_prefix(self, slab: np.ndarray, stop: int):
         out = np.zeros(1, dtype=MODEL_DTYPE)

@@ -122,7 +122,7 @@ extern "C" MG_API void mg_pool_trim(void)
 	cudaSetDevice(device);
 }
 
-extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 1u; }
+extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 2u; }
 
 struct mg_comm_state;
 
@@ -146,6 +146,8 @@ struct mg_ctx {
 	FindLimits limits{0, 0};          // mg_ctx_set_finder_limits (0, 0 = the reference's unbounded enumeration)
 	double last_encode_ms = 0;        // mg_encode_slab*: device time and events of the last call
 	unsigned long long last_encode_events = 0;
+	double last_decode_ms = 0;        // mg_decode_stream: device time and events of the last call
+	unsigned long long last_decode_events = 0;
 };
 
 struct DevBuf {
@@ -742,6 +744,87 @@ extern "C" MG_API int mg_encode_slab_buffer(mg_ctx* ctx, const LZMAPacket* slab,
 	if (*out_len > cap) return fail(MG_EINVAL, "mg_encode_slab_buffer: need %zu bytes, have %zu", *out_len, cap);
 	make_header(ctx, out);
 	memcpy(out + 13, payload.data(), payload.size());
+	return MG_OK;
+}
+
+// ---- stream -> slab ------------------------------------------------------------------------------------
+static const char* decode_error(uint32_t err)
+{
+	switch (err) {
+	case DEC_FIRST_BYTE: return "the range coder's first byte is not 0";
+	case DEC_LITERAL: return "a literal differs from the input";
+	case DEC_SOURCE: return "a match or rep reaches before position 0";
+	case DEC_PAST_END: return "a packet runs past the end of the input";
+	case DEC_COPY: return "a match or rep copies bytes that differ from the input";
+	case DEC_MARKER: return "an end marker where none may stand";
+	case DEC_SHORT: return "the stream ends before the input does";
+	case DEC_TRAILING: return "bytes follow the last packet";
+	case DEC_CODE: return "the range decoder does not end at code 0";
+	default: return "unknown";
+	}
+}
+
+extern "C" MG_API int mg_decode_stream(mg_ctx* ctx, const uint8_t* stream, size_t len, LZMAPacket* out_slab)
+{
+	if (!ctx || !stream || !out_slab) return fail(MG_EINVAL, "mg_decode_stream: null argument");
+	if (len < 13 + 5) return fail(MG_EINVAL, "mg_decode_stream: %zu bytes are shorter than any LZMA-alone stream", len);
+	if (stream[0] != 0) {
+		const unsigned props = stream[0];
+		return fail(MG_EINVAL, "mg_decode_stream: properties byte %u (lc = %u, lp = %u, pb = %u); only lc = lp = pb = 0 is supported",
+		            props, props % 9, props / 9 % 5, props / 45);
+	}
+	uint64_t size = 0;
+	for (int i = 0; i < 8; i++) size |= (uint64_t)stream[5 + i] << (8 * i);
+	const bool known = size != ~0ull;
+	if (known && size != ctx->n)
+		return fail(MG_EINVAL, "mg_decode_stream: the stream is of %llu bytes, the input of %u", (unsigned long long)size, ctx->n);
+	CU(cudaSetDevice(ctx->device));
+	const uint32_t n = ctx->n;
+	const size_t payload = len - 13;
+	DevBuf dstream, slab, status;
+	if (int rc = dev_alloc(dstream, payload)) return rc;
+	if (int rc = dev_alloc(slab, (size_t)n * 8)) return rc;
+	if (int rc = dev_alloc(status, sizeof(DecodeStatus))) return rc;
+	CU(cudaMemcpyAsync(dstream.p, stream + 13, payload, cudaMemcpyHostToDevice, ctx->stream));
+	fill_literal_kernel<<<grid_for(n, 256, ctx->sm_count * 8), 256, 0, ctx->stream>>>(slab.as<uint64_t>(), n);
+	CU(cudaGetLastError());
+	DecodeArgs a;
+	a.data = ctx->d_data;
+	a.n = n;
+	a.stream = dstream.as<uint8_t>();
+	a.len = payload;
+	a.known_size = known ? 1u : 0u;
+	a.slab = slab.as<uint64_t>();
+	a.status = status.as<DecodeStatus>();
+	cudaEvent_t t0, t1;
+	CU(cudaEventCreate(&t0));
+	CU(cudaEventCreate(&t1));
+	CU(cudaEventRecord(t0, ctx->stream));
+	decode_kernel<<<1, 32, 0, ctx->stream>>>(a);
+	CU(cudaEventRecord(t1, ctx->stream));
+	CU(cudaGetLastError());
+	DecodeStatus st;
+	CU(cudaMemcpyAsync(&st, status.p, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	{
+		float ms = 0;
+		cudaEventElapsedTime(&ms, t0, t1);
+		ctx->last_decode_ms = ms;
+		ctx->last_decode_events = st.events;
+		cudaEventDestroy(t0);
+		cudaEventDestroy(t1);
+	}
+	if (st.err != DEC_OK)
+		return fail(MG_ESLAB, "mg_decode_stream: position %u: %s (%llu of %zu payload bytes read)", st.pos, decode_error(st.err),
+		            st.consumed, payload);
+	return download_unpacked(ctx, slab.as<uint64_t>(), n, out_slab);
+}
+
+extern "C" MG_API int mg_decode_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* events)
+{
+	if (!ctx) return fail(MG_EINVAL, "mg_decode_stats: null context");
+	if (kernel_ms) *kernel_ms = ctx->last_decode_ms;
+	if (events) *events = ctx->last_decode_events;
 	return MG_OK;
 }
 

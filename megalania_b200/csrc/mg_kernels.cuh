@@ -2290,4 +2290,290 @@ __global__ void index_scatter_kernel(const uint8_t* __restrict__ data, uint32_t 
 	index_walk(data, n, rows + (size_t)wid * INDEX_KEYS, begin, end, start, occ);
 }
 
+// ---- K6: LZMA-alone payload -> slab (the range coder of K5 run backwards) ---------------------------------
+// Range decoding is one dependent chain, so one warp: lane 0 decodes, the warp checks a match's bytes against the
+// resident input 32 at a time.  The model is the reference's plain one (src/lzma_state.h:15-55, the order
+// export_model maps to) with plain probabilities: the walk's bank-owned slot map and transition tables serve
+// lane-parallel pricing, which a decoder has no use for.  Every decoded byte is compared with the input instead of
+// being written, so a stream either decodes to exactly this input or is rejected with the position it failed at.
+constexpr uint32_t DS_LIT = 0, DS_LEN = 768, DS_REPLEN = DS_LEN + 514, DS_POSSLOT = DS_REPLEN + 514;
+constexpr uint32_t DS_ALIGN = DS_POSSLOT + 256, DS_POSCODER = DS_ALIGN + 16, DS_ISMATCH = DS_POSCODER + 115;
+constexpr uint32_t DS_ISREP = DS_ISMATCH + 192, DS_ISREPG0 = DS_ISREP + 12, DS_ISREPG1 = DS_ISREPG0 + 12;
+constexpr uint32_t DS_ISREPG2 = DS_ISREPG1 + 12, DS_ISREP0LONG = DS_ISREPG2 + 12, DS_TOTAL = DS_ISREP0LONG + 192;
+constexpr uint32_t DL_CHOICE2 = 1, DL_LOW = 2, DL_MID = 2 + 128, DL_HIGH = 2 + 256;  // one length coder, pos_state 0
+static_assert(DS_TOTAL == 2615, "the decoder's model is the reference's");
+
+// what stopped the decoder (DecodeStatus.err); 0 = the stream is this input's
+enum : uint32_t {
+	DEC_OK = 0,
+	DEC_FIRST_BYTE = 1,  // the range coder's first byte is not 0
+	DEC_LITERAL = 2,     // a literal differs from the input
+	DEC_SOURCE = 3,      // a match or rep reaches before position 0
+	DEC_PAST_END = 4,    // a packet runs past the input's end (or a packet where only the end marker may stand)
+	DEC_COPY = 5,        // a match or rep copies bytes that differ from the input
+	DEC_MARKER = 6,      // an end marker before the input's end, or in a stream whose size is known
+	DEC_SHORT = 7,       // the stream ends before the input does
+	DEC_TRAILING = 8,    // bytes left over after the last packet
+	DEC_CODE = 9         // the range decoder's code is not 0 at the end
+};
+
+struct DecodeStatus {
+	uint32_t err;
+	uint32_t pos;                 // position of the packet that failed (n when the end checks failed)
+	unsigned long long events;    // modelled bits + direct-bit groups decoded
+	unsigned long long consumed;  // payload bytes read
+};
+
+struct DecodeArgs {
+	const uint8_t* data;     // the context's input (n + 32 bytes, zero padded)
+	uint32_t n;
+	const uint8_t* stream;   // the payload: everything after the 13-byte header
+	unsigned long long len;  // its length
+	uint32_t known_size;     // 1: stop at n; 0: the end marker must stand at n
+	uint64_t* slab;          // n packed slots, filled with PK_LITERAL beforehand
+	DecodeStatus* status;
+};
+
+constexpr uint32_t DEC_BUF = 16384;   // payload bytes staged in shared memory
+constexpr uint32_t DEC_MARGIN = 256;  // restage when fewer are left: a packet reads at most 48 (one per bit, <= 48 bits)
+
+struct RangeDecoder {
+	uint16_t* probs;
+	const uint8_t* buf;           // staged payload [base, base + DEC_BUF)
+	unsigned long long base, at, len;
+	uint32_t range, code;
+	uint32_t short_read;
+	unsigned long long events;
+};
+
+__device__ __forceinline__ void rd_shift(RangeDecoder& d)
+{
+	d.range <<= 8;
+	uint32_t b = 0;
+	if (d.at < d.len && d.at - d.base < DEC_BUF) b = d.buf[d.at++ - d.base];
+	else d.short_read = 1;
+	d.code = (d.code << 8) | b;
+}
+
+// src/range_encoder.c:47-64 and src/probability_model.c:5-15, backwards
+__device__ __forceinline__ uint32_t rd_bit(RangeDecoder& d, uint32_t slot)
+{
+	uint32_t v = d.probs[slot];
+	const uint32_t bound = (d.range >> 11) * v;
+	uint32_t bit;
+	if (d.code < bound) {
+		d.range = bound;
+		v += (2048u - v) >> 5;
+		bit = 0;
+	} else {
+		d.code -= bound;
+		d.range -= bound;
+		v -= v >> 5;
+		bit = 1;
+	}
+	d.probs[slot] = (uint16_t)v;
+	d.events++;
+	if ((d.range & 0xFF000000u) == 0) rd_shift(d);  // p stays within [31, 2017]: one shift always suffices
+	return bit;
+}
+
+// src/range_encoder.c:66-81, backwards
+__device__ __forceinline__ uint32_t rd_direct(RangeDecoder& d, uint32_t nbits)
+{
+	uint32_t value = 0;
+	d.events++;
+	while (nbits--) {
+		d.range >>= 1;
+		const uint32_t bit = d.code >= d.range ? 1u : 0u;
+		if (bit) d.code -= d.range;
+		value = (value << 1) | bit;
+		if ((d.range & 0xFF000000u) == 0) rd_shift(d);
+	}
+	return value;
+}
+
+__device__ __forceinline__ uint32_t rd_tree(RangeDecoder& d, uint32_t base, uint32_t nbits)
+{
+	uint32_t node = 1;
+	for (uint32_t i = 0; i < nbits; i++) node = (node << 1) | rd_bit(d, base + node);
+	return node - (1u << nbits);
+}
+
+__device__ __forceinline__ uint32_t rd_tree_rev(RangeDecoder& d, uint32_t base, uint32_t nbits)
+{
+	uint32_t node = 1, value = 0;
+	for (uint32_t i = 0; i < nbits; i++) {
+		const uint32_t bit = rd_bit(d, base + node);
+		node = (node << 1) | bit;
+		value |= bit << i;
+	}
+	return value;
+}
+
+// src/lzma_packet_encoder.c:42-63
+__device__ __forceinline__ uint32_t rd_length(RangeDecoder& d, uint32_t base)
+{
+	if (!rd_bit(d, base)) return 2 + rd_tree(d, base + DL_LOW, 3);
+	if (!rd_bit(d, base + DL_CHOICE2)) return 10 + rd_tree(d, base + DL_MID, 3);
+	return 18 + rd_tree(d, base + DL_HIGH, 8);
+}
+
+// src/lzma_packet_encoder.c:71-104: distance - 1 (0xffffffff = the end marker)
+__device__ __forceinline__ uint32_t rd_distance(RangeDecoder& d, uint32_t len)
+{
+	const uint32_t lctx = len - 2 < 3 ? len - 2 : 3;
+	const uint32_t pslot = rd_tree(d, DS_POSSLOT + lctx * 64, 6);
+	if (pslot < 4) return pslot;
+	const uint32_t nlow = (pslot >> 1) - 1;
+	const uint32_t dist = (2u | (pslot & 1u)) << nlow;
+	if (pslot < 14) return dist + rd_tree_rev(d, DS_POSCODER + dist - pslot, nlow);
+	const uint32_t mid = rd_direct(d, nlow - 4) << 4;
+	return dist + mid + rd_tree_rev(d, DS_ALIGN, 4);
+}
+
+__global__ void __launch_bounds__(32) decode_kernel(DecodeArgs a)
+{
+	__shared__ uint16_t probs[DS_TOTAL];
+	__shared__ __align__(16) uint8_t buf[DEC_BUF];
+	const uint32_t lane = threadIdx.x;
+	for (uint32_t i = lane; i < DS_TOTAL; i += 32) probs[i] = 1024;  // src/probability.h:7
+	RangeDecoder d;
+	d.probs = probs;
+	d.buf = buf;
+	d.base = 0;
+	d.at = 0;
+	d.len = a.len;
+	d.range = 0xFFFFFFFFu;
+	d.code = 0;
+	d.short_read = 0;
+	d.events = 0;
+	const unsigned long long first = a.len < DEC_BUF ? a.len : DEC_BUF;
+	for (uint32_t i = lane; i < first; i += 32) buf[i] = a.stream[i];
+	__syncwarp();
+	uint32_t err = DEC_OK, pos = 0;
+	// lane 0's decoder state: the automaton and the rep distances (src/lzma_state.c)
+	uint32_t ctx = 0, rep0 = 0, rep1 = 0, rep2 = 0, rep3 = 0;
+	if (lane == 0) {
+		if (a.len < 5) {
+			err = DEC_SHORT;
+		} else if (buf[0] != 0) {
+			err = DEC_FIRST_BYTE;
+		} else {
+			for (int i = 1; i < 5; i++) d.code = (d.code << 8) | buf[i];
+			d.at = 5;
+		}
+	}
+	err = __shfl_sync(FULL, err, 0);
+	while (err == DEC_OK) {
+		if (a.known_size && pos == a.n) break;
+		// restage the payload when the next packet could read past the staged bytes
+		const unsigned long long at = __shfl_sync(FULL, d.at, 0);
+		if (at + DEC_MARGIN > d.base + DEC_BUF && d.base + DEC_BUF < a.len) {
+			__syncwarp();
+			const unsigned long long left = a.len - at;
+			const uint32_t count = left < DEC_BUF ? (uint32_t)left : DEC_BUF;
+			for (uint32_t i = lane; i < count; i += 32) buf[i] = a.stream[at + i];
+			d.base = at;
+			__syncwarp();
+		}
+		uint32_t type = T_LITERAL, len = 1, dist = 0, src = 0, marker = 0;  // src: distance - 1 of the bytes a copy reads
+		if (lane == 0) {
+			if (d.short_read) {
+				err = DEC_SHORT;
+			} else if (!rd_bit(d, DS_ISMATCH + (ctx << 4))) {
+				// src/lzma_packet_encoder.c:106-136: the matched tree while the decoded bits agree with the match byte
+				if (pos >= a.n) {
+					err = DEC_PAST_END;
+				} else {
+					bool matched = ctx >= 7;
+					const uint32_t mbyte = matched && pos > rep0 ? a.data[pos - rep0 - 1] : 0u;
+					uint32_t node = 1;
+					for (int i = 7; i >= 0; i--) {
+						const uint32_t mbit = (mbyte >> i) & 1u;
+						const uint32_t slot = matched ? node + ((1u + mbit) << 8) : node;
+						const uint32_t bit = rd_bit(d, DS_LIT + slot);
+						matched = matched && mbit == bit;
+						node = (node << 1) | bit;
+					}
+					if ((node & 0xffu) != a.data[pos]) err = DEC_LITERAL;
+				}
+			} else if (!rd_bit(d, DS_ISREP + ctx)) {
+				len = rd_length(d, DS_LEN);
+				dist = rd_distance(d, len);
+				if (dist == 0xFFFFFFFFu) {
+					if (a.known_size || pos != a.n) err = DEC_MARKER;
+					marker = 1;
+				} else {
+					type = T_MATCH;
+					src = dist;
+				}
+			} else if (!rd_bit(d, DS_ISREPG0 + ctx)) {
+				src = rep0;
+				if (!rd_bit(d, DS_ISREP0LONG + (ctx << 4))) {
+					type = T_SHORT_REP;
+				} else {
+					type = T_LONG_REP;
+					len = rd_length(d, DS_REPLEN);
+				}
+			} else {
+				dist = 1;
+				if (rd_bit(d, DS_ISREPG1 + ctx)) dist = rd_bit(d, DS_ISREPG2 + ctx) ? 3 : 2;
+				type = T_LONG_REP;
+				len = rd_length(d, DS_REPLEN);
+				src = dist == 1 ? rep1 : dist == 2 ? rep2 : rep3;
+			}
+			if (err == DEC_OK && !marker && type != T_LITERAL) {
+				if ((unsigned long long)pos < (unsigned long long)src + 1) err = DEC_SOURCE;
+				else if ((unsigned long long)pos + len > a.n) err = DEC_PAST_END;
+			}
+			if (err == DEC_OK && !marker) {
+				// src/lzma_state.c:29-81: the automaton and the rep distances
+				if (type == T_MATCH) {
+					rep3 = rep2;
+					rep2 = rep1;
+					rep1 = rep0;
+					rep0 = dist;
+				} else if (type == T_LONG_REP && dist != 0) {
+					if (dist == 3) rep3 = rep2;
+					if (dist >= 2) rep2 = rep1;
+					rep1 = rep0;
+					rep0 = src;
+				}
+				ctx = type == T_LITERAL ? (ctx < 4 ? 0u : ctx < 10 ? ctx - 3 : ctx - 6)
+				    : type == T_MATCH   ? (ctx < 7 ? 7u : 10u)
+				    : type == T_SHORT_REP ? (ctx < 7 ? 9u : 11u)
+				                          : (ctx < 7 ? 8u : 11u);
+			}
+		}
+		err = __shfl_sync(FULL, err, 0);
+		marker = __shfl_sync(FULL, marker, 0);
+		if (err != DEC_OK || marker) break;
+		type = __shfl_sync(FULL, type, 0);
+		len = __shfl_sync(FULL, len, 0);
+		src = __shfl_sync(FULL, src, 0);
+		if (type != T_LITERAL) {
+			// the copied bytes must be the input's, 32 per step
+			bool differ = false;
+			for (uint32_t i = lane; i < len; i += 32) differ |= a.data[pos + i] != a.data[pos - src - 1 + i];
+			if (__any_sync(FULL, differ)) {
+				err = DEC_COPY;
+				break;
+			}
+		}
+		if (lane == 0) a.slab[pos] = pk_pack(type, dist, len);
+		pos += len;
+	}
+	if (lane == 0) {
+		if (err == DEC_OK) {
+			if (d.short_read) err = DEC_SHORT;
+			else if (d.at != a.len) err = DEC_TRAILING;
+			else if (d.code != 0) err = DEC_CODE;
+		}
+		a.status->err = err;
+		a.status->pos = pos;
+		a.status->events = d.events;
+		a.status->consumed = d.at;
+	}
+}
+
 }  // namespace mg

@@ -15,6 +15,10 @@
  * --gpus N runs one host thread, one context and one chain population per GPU; the ranks meet between
  * epochs / rounds through the library's NCCL collectives (mg_comm_*): best-slab broadcast in the epoch
  * schedule, region merge by all-reduce in the cooperative one.  No Python, no torch.
+ *
+ * --resume FILE starts the search from the slab of an .lzma stream of the same input (an earlier output, or
+ * liblzma's with lc = lp = pb = 0), decoded on the device by mg_decode_stream, instead of from zero; the run
+ * never writes a slab costlier than the one it read.
  */
 #include <pthread.h>
 #include <stdio.h>
@@ -30,7 +34,7 @@ static void usage(const char* argv0)
 	fprintf(stderr,
 	        "usage: %s [--chains N] [--iters N] [--epochs N] [--steps N] [--seed N] [--device N] [--gpus N] [--top-k N]\n"
 	        "          [--rounds N | --time SECONDS] [--round-ms N] [--group N] [--temp T] [--sm-khz N]\n"
-	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS] filename\n",
+	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS | --resume FILE] filename\n",
 	        argv0);
 }
 
@@ -39,6 +43,8 @@ typedef struct {
 	unsigned long long seed;
 	const uint8_t* data;
 	size_t size;
+	const uint8_t* resume; /* --resume: the .lzma stream to start from, NULL = none */
+	size_t resume_size;
 } Config;
 
 typedef struct {
@@ -53,6 +59,8 @@ typedef struct {
 	LZMAPacket* packets_best;
 	int have_best;
 	uint64_t best_perplexity;
+	LZMAPacket* resumed;     /* --resume: the decoded slab and its cost */
+	uint64_t resumed_cost;
 } Worker;
 
 static int die(const Worker* w, const char* what)
@@ -106,7 +114,7 @@ static int run_rounds(Worker* w, mg_anneal* an)
 		fprintf(stderr, "out of memory\n");
 		return -1;
 	}
-	if (mg_anneal_set_slab(an, 0, chains, NULL, 1, 1)) return die(w, "mg_anneal_set_slab");
+	if (mg_anneal_set_slab(an, 0, chains, w->resumed, 1, 1)) return die(w, "mg_anneal_set_slab");
 	if (c->greedy) {
 		/* --greedy N: start from a greedy parse of N regions instead of the all-literal slab; every rank builds
 		 * the same slab (the parse draws nothing) */
@@ -191,7 +199,13 @@ static int run_rounds(Worker* w, mg_anneal* an)
 			fprintf(stderr, "current file size: %f\tround: %u/%u - %s, %llu evals, %.0f evals/s\n", 18 + w->best_perplexity / 16384.f,
 			        r + 1, c->rounds, kept, total_evals, total_evals / (device_ms / 1e3));
 	}
-	if (mg_anneal_get_slab(an, 0, 0, w->packets_best)) return die(w, "mg_anneal_get_slab");
+	if (w->resumed && w->resumed_cost <= w->best_perplexity) {
+		/* the rounds ended no cheaper than the resumed slab: keep that one */
+		memcpy(w->packets_best, w->resumed, sizeof(LZMAPacket) * file_size);
+		w->best_perplexity = w->resumed_cost;
+	} else if (mg_anneal_get_slab(an, 0, 0, w->packets_best)) {
+		return die(w, "mg_anneal_get_slab");
+	}
 	w->have_best = 1;
 	free(bounds);
 	free(owners);
@@ -219,8 +233,8 @@ static int run_epochs(Worker* w, mg_anneal* an)
 	for (unsigned step = 0; step < c->steps; step++) {
 		for (unsigned epoch = 0; epoch < c->epochs; epoch++) {
 			/* src/main.c:71-77: fresh slab in step 0, the best so far afterwards; cost 0 means
-			 * "first proposal always accepted" */
-			if (mg_anneal_set_slab(an, 0, chains, (step != 0 && w->have_best) ? w->packets_best : NULL, 0, 0))
+			 * "first proposal always accepted".  A resumed run starts step 0 from the resumed slab */
+			if (mg_anneal_set_slab(an, 0, chains, ((step != 0 || w->resumed) && w->have_best) ? w->packets_best : NULL, 0, 0))
 				return die(w, "mg_anneal_set_slab");
 			mg_anneal_run_params run;
 			memset(&run, 0, sizeof(run));
@@ -268,6 +282,34 @@ static int run_epochs(Worker* w, mg_anneal* an)
 	return 0;
 }
 
+/* --resume: every rank decodes the stream on its own context (deterministic: all ranks hold the same slab) and
+ * scores it; it becomes the best so far */
+static int resume_from_stream(Worker* w)
+{
+	const Config* c = w->cfg;
+	w->resumed = malloc(sizeof(LZMAPacket) * c->size);
+	w->packets_best = malloc(sizeof(LZMAPacket) * c->size);
+	if (!w->resumed || !w->packets_best) {
+		fprintf(stderr, "out of memory\n");
+		return -1;
+	}
+	if (mg_decode_stream(w->ctx, c->resume, c->resume_size, w->resumed)) {
+		/* a stream of another input is a usage error on every rank alike: leave before any collective */
+		fprintf(stderr, "[gpu %u] mg_decode_stream: %s\n", c->device + (unsigned)w->rank, mg_last_error());
+		if (c->gpus > 1) {
+			fflush(stderr);
+			_exit(255);
+		}
+		return -1;
+	}
+	if (mg_score_slabs(w->ctx, w->resumed, 1, &w->resumed_cost)) return die(w, "mg_score_slabs");
+	memcpy(w->packets_best, w->resumed, sizeof(LZMAPacket) * c->size);
+	w->best_perplexity = w->resumed_cost;
+	w->have_best = 1;
+	if (w->rank == 0) fprintf(stderr, "current file size: %f\tresumed (%zu-byte stream)\n", 18 + w->resumed_cost / 16384.f, c->resume_size);
+	return 0;
+}
+
 static void* worker_main(void* arg)
 {
 	Worker* w = (Worker*)arg;
@@ -281,6 +323,7 @@ static void* worker_main(void* arg)
 			die(w, "mg_ctx_create");
 			break;
 		}
+		if (c->resume && resume_from_stream(w) != 0) break;
 		/* SM clocks per millisecond: the device's own figure (mg_ctx_sm_clock_khz) unless --sm-khz says otherwise;
 		 * 1965 MHz (B200) only if the driver reports nothing */
 		w->sm_khz = c->sm_khz ? c->sm_khz : mg_ctx_sm_clock_khz(w->ctx);
@@ -303,7 +346,7 @@ static void* worker_main(void* arg)
 			die(w, "mg_anneal_create");
 			break;
 		}
-		w->packets_best = malloc(sizeof(LZMAPacket) * c->size);
+		if (!w->packets_best) w->packets_best = malloc(sizeof(LZMAPacket) * c->size);
 		if (!w->packets_best) {
 			fprintf(stderr, "out of memory\n");
 			break;
@@ -332,6 +375,7 @@ int main(int argc, char** argv)
 	cfg.seed = 1673551;  /* src/main.c:68 */
 	unsigned time_s = 0; /* --time: annealing budget in seconds of SM time */
 	const char* filename = NULL;
+	const char* resume_name = NULL;
 	for (int i = 1; i < argc; i++) {
 		const char* a = argv[i];
 		unsigned* target = NULL;
@@ -357,6 +401,9 @@ int main(int argc, char** argv)
 		} else if (!strcmp(a, "--seed")) {
 			if (++i >= argc) { usage(argv[0]); return -1; }
 			cfg.seed = strtoull(argv[i], NULL, 10);
+		} else if (!strcmp(a, "--resume")) {
+			if (++i >= argc) { usage(argv[0]); return -1; }
+			resume_name = argv[i];
 		} else if (a[0] == '-' && a[1] == '-') {
 			usage(argv[0]);
 			return -1;
@@ -369,7 +416,7 @@ int main(int argc, char** argv)
 	}
 	if (time_s > 0 && cfg.round_ms > 0) cfg.rounds = (time_s * 1000u + cfg.round_ms - 1) / cfg.round_ms;
 	if (filename == NULL || cfg.chains == 0 || cfg.gpus == 0 || cfg.gpus > 64 ||
-	    (cfg.rounds == 0 && (cfg.steps == 0 || cfg.epochs == 0))) {
+	    (cfg.rounds == 0 && (cfg.steps == 0 || cfg.epochs == 0)) || (resume_name && cfg.greedy)) {
 		usage(argv[0]);
 		return -1;
 	}
@@ -388,6 +435,12 @@ int main(int argc, char** argv)
 	if (input_file_open(&input, filename) < 0) return -1;
 	cfg.data = input.data;
 	cfg.size = input.size;
+	InputFile resume_file = { NULL, 0 };
+	if (resume_name) {
+		if (input_file_open(&resume_file, resume_name) < 0) return -1;
+		cfg.resume = resume_file.data;
+		cfg.resume_size = resume_file.size;
+	}
 	if (cfg.iters == 0) cfg.iters = cfg.size < 2000 ? (unsigned)cfg.size : 2000;
 
 	Worker* workers = calloc(cfg.gpus, sizeof(Worker));
@@ -448,10 +501,12 @@ int main(int argc, char** argv)
 
 	for (unsigned r = 0; r < cfg.gpus; r++) {
 		free(workers[r].packets_best);
+		free(workers[r].resumed);
 		mg_ctx_destroy(workers[r].ctx);
 	}
 	free(workers);
 	free(threads);
+	if (resume_name) input_file_close(&resume_file);
 	input_file_close(&input);
 	return 0;
 }
