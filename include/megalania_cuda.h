@@ -271,6 +271,29 @@ MG_API int mg_anneal_set_slab(mg_anneal* an, uint32_t first, uint32_t count, con
  * oracle's greedy parse packet for packet.  Search strategy on top of the hot path: off unless asked for. */
 MG_API int mg_anneal_greedy_init(mg_anneal* an, uint32_t nregions, uint32_t dst_chain, uint64_t* cost_out);
 
+/* A starting slab from a shortest-path parse instead of a greedy one (no reference counterpart; liblzma's optimum
+ * parse makes the same approximations).  Regions as in mg_anneal_greedy_init (equal cuts, at least 64 bytes each),
+ * each parsed from a fresh model; the context's finder limits do not apply.
+ *   Match list of position i (0 < i < n - 1): the bigram bucket of (d[i], d[i+1]) walked from the nearest earlier
+ *   occurrence backwards, at most max_occ occurrences (0 = 64), each extended up to min(273, n - i) bytes; an
+ *   occurrence becomes an entry (len, distance - 1) only when it is longer than every earlier entry, and the walk
+ *   stops at an entry of min(273, n - i) bytes or at 32 entries.  A MATCH of length l uses the first entry with
+ *   len >= l (the nearest distance that reaches l).
+ *   Parse of one region, one exact adaptive model: blocks of B = min(4096, bytes left) from the current position p.
+ *   Prices come from the model as it stands at p.  Node 0 holds cost 0 and the model's automaton state and rep
+ *   distances; node j keeps the cheapest packet that reached it and the state after it.  Nodes are relaxed in
+ *   ascending j, edges in the order LITERAL (matched against rep0 after a match or rep), SHORT_REP, then for each
+ *   length l = 2..min(273, B - j): LONG_REP 0..3 (where that rep matches l bytes), MATCH; a target takes its
+ *   cheapest edge (the first on a tie) and only if that is strictly cheaper than what it holds.  The path that
+ *   reaches node B is written into the slab and the exact model runs through it; no packet crosses a block's end.
+ * The stitched slab goes through the same repair pass as mg_anneal_greedy_init's, which prices it exactly
+ * (*cost_out).  nregions = 1 is the CPU parse of the tests packet for packet.  Off unless asked for. */
+MG_API int mg_anneal_optimal_init(mg_anneal* an, uint32_t nregions, uint32_t max_occ, uint32_t dst_chain,
+                                  uint64_t* cost_out);
+/* Device time (CUDA events around the match-list and parse kernels) and nodes relaxed (bytes parsed) by the last
+ * mg_anneal_optimal_init on ctx. */
+MG_API int mg_optimal_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* nodes);
+
 /* Cooperative regions.  After region-confined chains (mg_anneal_run_params.regions) have run from a
  * common slab, builds the slab that takes region r = [bounds[r], bounds[r+1]) from chain owners[r]
  * (bounds[0] = 0, bounds[nregions] = n), stores it as the current slab of chain `dst_chain`, repairs the

@@ -6,6 +6,7 @@ The names follow the reference's vocabulary (slab, packet, top-k finder, perplex
   Context.find_topk(...)        top_k_packet_finder_find + pop loop         (src/top_k_packet_finder.c)
   Context.encode_slab(slab)     header + range_encoder pass                 (src/main.c:110-119)
   Context.decode_stream(stream) .lzma stream (lc = lp = pb = 0) -> slab, to resume a search (no reference counterpart)
+  Annealer.optimal_init(...)    shortest-path parse as a starting slab                           (no reference counterpart)
   Annealer(ctx, chains, ...)    the loop of src/main.c:78-102 on many chains
 
 There is no CPU path: importing works anywhere, but every compute call needs the CUDA library
@@ -88,7 +89,7 @@ EXPORTS = [
     "mg_comm_unique_id", "mg_comm_init", "mg_comm_destroy", "mg_comm_rank", "mg_comm_size", "mg_comm_exchange_best",
     "mg_comm_temper_exchange", "mg_temper_decide", "mg_comm_merge_regions", "mg_comm_stats", "mg_pool_trim",
     "mg_comm_broadcast_chain", "mg_comm_allgather_u64", "mg_ctx_set_finder_limits", "mg_anneal_greedy_init",
-    "mg_decode_stream", "mg_decode_stats",
+    "mg_decode_stream", "mg_decode_stats", "mg_anneal_optimal_init", "mg_optimal_stats",
 ]
 
 _lib = None
@@ -170,6 +171,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mg_encode_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
     L.mg_decode_stream.argtypes = [vp, vp, sz, vp]
     L.mg_decode_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
+    L.mg_anneal_optimal_init.argtypes = [vp, u32, u32, u32, C.POINTER(u64)]
+    L.mg_optimal_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
     _lib = L
     return L
 
@@ -305,6 +308,12 @@ class Context:
         ms, ev = C.c_double(0), C.c_uint64(0)
         _check(self._lib.mg_decode_stats(self._h, C.byref(ms), C.byref(ev)))
         return {"kernel_ms": ms.value, "events": int(ev.value)}
+
+    def optimal_stats(self) -> dict:
+        """Device time of the last Annealer.optimal_init's match-list and parse kernels, and the nodes it relaxed."""
+        ms, nodes = C.c_double(0), C.c_uint64(0)
+        _check(self._lib.mg_optimal_stats(self._h, C.byref(ms), C.byref(nodes)))
+        return {"kernel_ms": ms.value, "nodes": int(nodes.value)}
 
     def model_after_prefix(self, slab: np.ndarray, stop: int):
         out = np.zeros(1, dtype=MODEL_DTYPE)
@@ -509,6 +518,14 @@ class Annealer:
         into chain dst_chain; returns its cost.  One region, no finder limits = the oracle's greedy slab."""
         cost = C.c_uint64(0)
         _check(self._lib.mg_anneal_greedy_init(self._h, nregions, dst_chain, C.byref(cost)))
+        return int(cost.value)
+
+    def optimal_init(self, nregions: int = 1, max_occ: int = 0, dst_chain: int = 0) -> int:
+        """mg_anneal_optimal_init: shortest-path parse of `nregions` byte regions side by side (match lists of at most
+        max_occ occurrences, 0 = 64), stitched, repaired and priced into chain dst_chain; returns its cost.  One
+        region = the CPU parse of the tests packet for packet."""
+        cost = C.c_uint64(0)
+        _check(self._lib.mg_anneal_optimal_init(self._h, nregions, max_occ, dst_chain, C.byref(cost)))
         return int(cost.value)
 
     def refresh_chain(self, chain: int, adopt_cost: bool = True) -> None:

@@ -122,7 +122,7 @@ extern "C" MG_API void mg_pool_trim(void)
 	cudaSetDevice(device);
 }
 
-extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 2u; }
+extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 3u; }
 
 struct mg_comm_state;
 
@@ -148,6 +148,8 @@ struct mg_ctx {
 	unsigned long long last_encode_events = 0;
 	double last_decode_ms = 0;        // mg_decode_stream: device time and events of the last call
 	unsigned long long last_decode_events = 0;
+	double last_optimal_ms = 0;       // mg_anneal_optimal_init: device time and nodes of the last call
+	unsigned long long last_optimal_nodes = 0;
 };
 
 struct DevBuf {
@@ -1500,6 +1502,84 @@ extern "C" MG_API int mg_anneal_greedy_init(mg_anneal* an, uint32_t nregions, ui
 	CU(cudaStreamSynchronize(ctx->stream));
 	if (herr) return fail(MG_ESLAB, "mg_anneal_greedy_init: %s", walk_error(herr));
 	return mg_anneal_merge_import(an, slab.p, abs.p, dst_chain, cost_out);
+}
+
+extern "C" MG_API int mg_anneal_optimal_init(mg_anneal* an, uint32_t nregions, uint32_t max_occ, uint32_t dst_chain,
+                                             uint64_t* cost_out)
+{
+	if (!an || dst_chain >= an->p.chains) return fail(MG_EINVAL, "mg_anneal_optimal_init: bad argument");
+	mg_ctx* ctx = an->ctx;
+	const uint32_t n = ctx->n;
+	if (nregions == 0) nregions = 1;
+	if (nregions > n / 64 + 1) nregions = n / 64 + 1;  // a region is at least 64 bytes
+	if (max_occ == 0) max_occ = 64;
+	CU(cudaSetDevice(ctx->device));
+	std::vector<uint32_t> bounds(nregions + 1);
+	for (uint32_t r = 0; r <= nregions; r++) bounds[r] = (uint32_t)((uint64_t)n * r / nregions);
+	// the parse's warps each keep one block of nodes (L2-resident scratch); regions are dealt over them
+	uint32_t blocks = (uint32_t)ctx->sm_count * 8;
+	if (blocks > nregions) blocks = nregions;
+	DevBuf slab, abs, dbounds, lists, counts, nodes, dnodes;
+	if (int rc = dev_alloc(slab, (size_t)n * 8)) return rc;
+	if (int rc = dev_alloc(abs, (size_t)n * 4)) return rc;
+	if (int rc = dev_alloc(dbounds, sizeof(uint32_t) * (nregions + 1))) return rc;
+	if (int rc = dev_alloc(lists, (size_t)n * OPT_LIST * sizeof(uint2))) return rc;
+	if (int rc = dev_alloc(counts, n)) return rc;
+	if (int rc = dev_alloc(nodes, (size_t)blocks * (OPT_BLOCK + 1) * 2 * sizeof(uint4))) return rc;
+	if (int rc = dev_alloc(dnodes, sizeof(unsigned long long))) return rc;
+	CU(cudaMemcpyAsync(dbounds.p, bounds.data(), sizeof(uint32_t) * (nregions + 1), cudaMemcpyHostToDevice, ctx->stream));
+	CU(cudaMemsetAsync(abs.p, 0, (size_t)n * 4, ctx->stream));
+	CU(cudaMemsetAsync(dnodes.p, 0, sizeof(unsigned long long), ctx->stream));
+	fill_literal_kernel<<<grid_for(n, 256, ctx->sm_count * 8), 256, 0, ctx->stream>>>(slab.as<uint64_t>(), n);
+	CU(cudaGetLastError());
+	MatchListArgs ml;
+	ml.data = ctx->d_data;
+	ml.n = n;
+	ml.occ_start = ctx->d_occ_start;
+	ml.occ = ctx->d_occ;
+	ml.max_occ = max_occ;
+	ml.lists = lists.as<uint2>();
+	ml.counts = counts.as<uint8_t>();
+	OptimalArgs o;
+	o.data = ctx->d_data;
+	o.n = n;
+	o.trans = ctx->d_trans;
+	o.lists = lists.as<uint2>();
+	o.counts = counts.as<uint8_t>();
+	o.bounds = dbounds.as<uint32_t>();
+	o.nregions = nregions;
+	o.nodes = nodes.as<uint4>();
+	o.slab = slab.as<uint64_t>();
+	o.abs_dist = abs.as<uint32_t>();
+	o.nodes_relaxed = dnodes.as<unsigned long long>();
+	cudaEvent_t t0, t1;
+	CU(cudaEventCreate(&t0));
+	CU(cudaEventCreate(&t1));
+	CU(cudaEventRecord(t0, ctx->stream));
+	matchlist_kernel<<<grid_for((size_t)n * 32, 256, ctx->sm_count * 64), 256, 0, ctx->stream>>>(ml);
+	optimal_kernel<<<blocks, 32, 0, ctx->stream>>>(o);
+	CU(cudaEventRecord(t1, ctx->stream));
+	CU(cudaGetLastError());
+	unsigned long long relaxed = 0;
+	CU(cudaMemcpyAsync(&relaxed, dnodes.p, sizeof(relaxed), cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	{
+		float ms = 0;
+		cudaEventElapsedTime(&ms, t0, t1);
+		ctx->last_optimal_ms = ms;
+		ctx->last_optimal_nodes = relaxed;
+		cudaEventDestroy(t0);
+		cudaEventDestroy(t1);
+	}
+	return mg_anneal_merge_import(an, slab.p, abs.p, dst_chain, cost_out);
+}
+
+extern "C" MG_API int mg_optimal_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* nodes)
+{
+	if (!ctx) return fail(MG_EINVAL, "mg_optimal_stats: null context");
+	if (kernel_ms) *kernel_ms = ctx->last_optimal_ms;
+	if (nodes) *nodes = ctx->last_optimal_nodes;
+	return MG_OK;
 }
 
 extern "C" MG_API int mg_anneal_broadcast_chain(mg_anneal* an, uint32_t src_chain)

@@ -2576,4 +2576,417 @@ __global__ void __launch_bounds__(32) decode_kernel(DecodeArgs a)
 	}
 }
 
+// ---- shortest-path parse (starting slabs, mg_anneal_optimal_init) ------------------------------------------
+// Semantics in include/megalania_cuda.h; tests/optimal_parse.c is the same parse with one region, written
+// sequentially.  Two kernels: the match list of every position (fully parallel), then one warp per region that
+// relaxes the nodes of a block in ascending order and commits the cheapest path.  The model is the reference's plain
+// one in shared memory (the DS_ slot map of K6): the parse reads it to build static price tables once per block and
+// adapts it once per committed packet, so the walk's lane-parallel layout would buy nothing here.
+constexpr uint32_t OPT_BLOCK = 4096;  // nodes per block (prices are those of the model at the block's start)
+constexpr uint32_t OPT_LIST = 32;     // match-list entries per position
+constexpr uint32_t OPT_INF = 0xffffffffu;
+
+// Match list of position i: walk the bigram bucket from the nearest earlier occurrence backwards (max_occ at most),
+// keep an entry only when it is longer than every earlier one, stop at min(273, n - i) bytes or at OPT_LIST entries.
+// One warp per position: 32 occurrences per step, their lengths byte by byte in the lanes, then the running maximum
+// over the lanes in walk order decides which become entries.
+struct MatchListArgs {
+	const uint8_t* data;
+	uint32_t n;
+	const uint32_t* occ_start;
+	const uint32_t* occ;
+	uint32_t max_occ;
+	uint2* lists;     // [n][OPT_LIST] (len, distance - 1)
+	uint8_t* counts;  // [n]
+};
+
+__global__ void __launch_bounds__(256) matchlist_kernel(MatchListArgs a)
+{
+	const uint32_t lane = threadIdx.x & 31;
+	const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+	for (uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < a.n; i += warps) {
+		uint32_t count = 0;
+		if (i != 0 && i + 1 < a.n) {
+			const uint32_t key = (uint32_t)a.data[i] << 8 | a.data[i + 1];
+			const uint32_t first = a.occ_start[key];
+			uint32_t lo = first, hi = a.occ_start[key + 1];
+			while (lo < hi) {  // the first occurrence at or after i (uniform: every lane searches alike)
+				const uint32_t mid = lo + (hi - lo) / 2;
+				if (a.occ[mid] < i) lo = mid + 1;
+				else hi = mid;
+			}
+			const uint32_t limit = a.n - i < 273 ? a.n - i : 273;
+			uint32_t best = 0, visited = 0, at = lo;
+			while (at > first && visited < a.max_occ && count < OPT_LIST && best < limit) {
+				uint32_t step = at - first < 32 ? at - first : 32;
+				if (a.max_occ - visited < step) step = a.max_occ - visited;
+				uint32_t len = 0, o = 0;
+				if (lane < step) {
+					o = a.occ[at - 1 - lane];
+					len = 2;
+					while (len < limit && a.data[i + len] == a.data[o + len]) len++;
+				}
+				uint32_t run = len;  // inclusive running maximum in walk order
+				for (uint32_t d = 1; d < 32; d <<= 1) {
+					const uint32_t v = __shfl_up_sync(FULL, run, d);
+					if (lane >= d && v > run) run = v;
+				}
+				uint32_t before = __shfl_up_sync(FULL, run, 1);
+				if (lane == 0) before = 0;
+				const bool keep = len > (before > best ? before : best);
+				const uint32_t mask = __ballot_sync(FULL, keep);
+				const uint32_t rank = count + __popc(mask & ((1u << lane) - 1u));
+				if (keep && rank < OPT_LIST) a.lists[(size_t)i * OPT_LIST + rank] = make_uint2(len, i - o - 1);
+				count += __popc(mask);
+				if (count > OPT_LIST) count = OPT_LIST;
+				const uint32_t top = __shfl_sync(FULL, run, 31);
+				if (top > best) best = top;
+				visited += step;
+				at -= step;
+			}
+		}
+		if (lane == 0) a.counts[i] = (uint8_t)count;
+	}
+}
+
+struct OptimalArgs {
+	const uint8_t* data;
+	uint32_t n;
+	const uint32_t* trans;    // the context's transition tables: section 0 holds the price of bit 0 at every p
+	const uint2* lists;       // matchlist_kernel's output
+	const uint8_t* counts;
+	const uint32_t* bounds;   // [nregions + 1]
+	uint32_t nregions;
+	uint4* nodes;             // [gridDim.x][OPT_BLOCK + 1][2]: (info, dist, rep0, rep1), (rep2, rep3, -, -)
+	uint64_t* slab;           // [n] packed, pre-filled with literals
+	uint32_t* abs_dist;       // [n] zeroed
+	unsigned long long* nodes_relaxed;
+};
+
+struct OptShared {
+	uint32_t price[2048];     // src/generate_table.py, the price of a bit against probability p
+	uint32_t cost[OPT_BLOCK + 1];
+	uint32_t lenp[2][274];    // match / rep length prices
+	uint32_t slotp[4][64];    // pos-slot prices per length context
+	uint32_t alignp[16];
+	uint32_t litp[256];       // plain-literal trees (without is_match)
+	uint32_t ent_len[OPT_LIST], ent_dist[OPT_LIST], ent_dp[OPT_LIST][4];
+	uint16_t probs[DS_TOTAL];
+};
+
+__device__ __forceinline__ uint32_t opt_bit(const OptShared& s, uint32_t slot, uint32_t bit)
+{
+	const uint32_t p = s.probs[slot];
+	return s.price[bit ? 2048u - p : p];
+}
+
+__device__ __forceinline__ uint32_t opt_tree(const OptShared& s, uint32_t base, uint32_t nbits, uint32_t value)
+{
+	uint32_t c = 0, node = 1;
+	for (uint32_t i = nbits; i-- > 0;) {
+		const uint32_t bit = (value >> i) & 1u;
+		c += opt_bit(s, base + node, bit);
+		node = (node << 1) | bit;
+	}
+	return c;
+}
+
+__device__ __forceinline__ uint32_t opt_tree_rev(const OptShared& s, uint32_t base, uint32_t nbits, uint32_t value)
+{
+	uint32_t c = 0, node = 1;
+	for (uint32_t i = 0; i < nbits; i++) {
+		const uint32_t bit = value & 1u;
+		c += opt_bit(s, base + node, bit);
+		node = (node << 1) | bit;
+		value >>= 1;
+	}
+	return c;
+}
+
+__device__ __forceinline__ uint32_t opt_length(const OptShared& s, uint32_t base, uint32_t len)
+{
+	uint32_t v = len - 2;
+	if (v < 8) return opt_bit(s, base, 0) + opt_tree(s, base + DL_LOW, 3, v);
+	v -= 8;
+	const uint32_t c = opt_bit(s, base, 1);
+	if (v < 8) return c + opt_bit(s, base + DL_CHOICE2, 0) + opt_tree(s, base + DL_MID, 3, v);
+	return c + opt_bit(s, base + DL_CHOICE2, 1) + opt_tree(s, base + DL_HIGH, 8, v - 8);
+}
+
+// adapt one slot (src/probability_model.c:5-15)
+__device__ __forceinline__ void opt_code(OptShared& s, uint32_t slot, uint32_t bit)
+{
+	uint32_t v = s.probs[slot];
+	if (bit) v -= v >> 5;
+	else v += (2048u - v) >> 5;
+	s.probs[slot] = (uint16_t)v;
+}
+
+__device__ __forceinline__ void opt_code_tree(OptShared& s, uint32_t base, uint32_t nbits, uint32_t value, bool rev)
+{
+	uint32_t node = 1;
+	for (uint32_t i = 0; i < nbits; i++) {
+		const uint32_t bit = rev ? (value >> i) & 1u : (value >> (nbits - 1 - i)) & 1u;
+		opt_code(s, base + node, bit);
+		node = (node << 1) | bit;
+	}
+}
+
+__device__ __forceinline__ void opt_code_length(OptShared& s, uint32_t base, uint32_t len)
+{
+	uint32_t v = len - 2;
+	opt_code(s, base, v >= 8);
+	if (v < 8) return opt_code_tree(s, base + DL_LOW, 3, v, false);
+	opt_code(s, base + DL_CHOICE2, v >= 16);
+	if (v < 16) return opt_code_tree(s, base + DL_MID, 3, v - 8, false);
+	opt_code_tree(s, base + DL_HIGH, 8, v - 16, false);
+}
+
+// the model's part of src/lzma_packet_encoder.c:106-194 for one packet (lane 0 only)
+__device__ void opt_code_packet(OptShared& s, const uint8_t* data, uint32_t pos, uint32_t ctx, uint32_t rep0,
+                                uint32_t type, uint32_t len, uint32_t dist)
+{
+	if (type == T_LITERAL) {
+		opt_code(s, DS_ISMATCH + (ctx << 4), 0);
+		const uint32_t byte = data[pos];
+		bool matched = ctx >= 7;
+		const uint32_t mbyte = matched ? data[pos - rep0 - 1] : 0u;
+		uint32_t node = 1;
+		for (int i = 7; i >= 0; i--) {
+			const uint32_t bit = (byte >> i) & 1u;
+			uint32_t slot = node;
+			if (matched) {
+				const uint32_t mbit = (mbyte >> i) & 1u;
+				slot += (1u + mbit) << 8;
+				matched = mbit == bit;
+			}
+			opt_code(s, DS_LIT + slot, bit);
+			node = (node << 1) | bit;
+		}
+		return;
+	}
+	opt_code(s, DS_ISMATCH + (ctx << 4), 1);
+	opt_code(s, DS_ISREP + ctx, type != T_MATCH);
+	if (type == T_MATCH) {
+		opt_code_length(s, DS_LEN, len);
+		const uint32_t lctx = len - 2 < 3 ? len - 2 : 3;
+		if (dist < 4) return opt_code_tree(s, DS_POSSLOT + lctx * 64, 6, dist, false);
+		const uint32_t nlow = 30u - (uint32_t)__clz(dist), low = dist & ((1u << nlow) - 1), high = dist >> nlow;
+		const uint32_t pslot = nlow * 2 + high;
+		opt_code_tree(s, DS_POSSLOT + lctx * 64, 6, pslot, false);
+		if (pslot < 14) opt_code_tree(s, DS_POSCODER + (high << nlow) - pslot, nlow, low, true);
+		else opt_code_tree(s, DS_ALIGN, 4, low & 15, true);
+		return;
+	}
+	if (type == T_SHORT_REP || dist == 0) {
+		opt_code(s, DS_ISREPG0 + ctx, 0);
+		opt_code(s, DS_ISREP0LONG + (ctx << 4), type == T_LONG_REP);
+	} else {
+		opt_code(s, DS_ISREPG0 + ctx, 1);
+		opt_code(s, DS_ISREPG1 + ctx, dist != 1);
+		if (dist != 1) opt_code(s, DS_ISREPG2 + ctx, dist != 2);
+	}
+	if (type == T_LONG_REP) opt_code_length(s, DS_REPLEN, len);
+}
+
+// node info word: type[7:0] | len[23:8] | ctx after the packet[31:24]
+__device__ __forceinline__ uint32_t opt_info(uint32_t type, uint32_t len, uint32_t ctx) { return type | (len << 8) | (ctx << 24); }
+
+// One warp per region, regions dealt over the CTAs.  Per node j (ascending), lane L owns the targets j + l with
+// l = L (mod 32): it takes the cheapest of its candidate edges (LITERAL, SHORT_REP for l = 1; LONG_REP 0..3, then
+// MATCH otherwise; the first one on a tie) and replaces the target only if that is strictly cheaper.  Being the only
+// writer of its targets within the step, it needs no atomics, and the result is the sequential rule.
+__global__ void __launch_bounds__(32) optimal_kernel(OptimalArgs a)
+{
+	__shared__ __align__(16) OptShared s;
+	const uint32_t lane = threadIdx.x;
+	for (uint32_t i = lane; i < 2048; i += 32) s.price[i] = i ? a.trans[i] >> 16 : 0u;
+	uint4* nodes = a.nodes + (size_t)blockIdx.x * (OPT_BLOCK + 1) * 2;
+	unsigned long long relaxed = 0;
+	for (uint32_t r = blockIdx.x; r < a.nregions; r += gridDim.x) {
+		const uint32_t lo = a.bounds[r], hi = a.bounds[r + 1];
+		for (uint32_t i = lane; i < DS_TOTAL; i += 32) s.probs[i] = 1024;  // src/probability.h:7
+		uint32_t ctx = 0, rep0 = 0, rep1 = 0, rep2 = 0, rep3 = 0;  // the exact model's state (every lane)
+		for (uint32_t p = lo; p < hi;) {
+			const uint32_t B = hi - p < OPT_BLOCK ? hi - p : OPT_BLOCK;
+			__syncwarp();
+			// static price tables from the model as it stands at p
+			for (uint32_t l = 2 + lane; l <= 273; l += 32) {
+				s.lenp[0][l] = opt_length(s, DS_LEN, l);
+				s.lenp[1][l] = opt_length(s, DS_REPLEN, l);
+			}
+			for (uint32_t i = lane; i < 256; i += 32) {
+				s.slotp[i >> 6][i & 63] = opt_tree(s, DS_POSSLOT + (i >> 6) * 64, 6, i & 63);
+				s.litp[i] = opt_tree(s, DS_LIT, 8, i);
+			}
+			if (lane < 16) s.alignp[lane] = opt_tree_rev(s, DS_ALIGN, 4, lane);
+			for (uint32_t j = lane; j <= B; j += 32) s.cost[j] = j ? OPT_INF : 0u;
+			if (lane == 0) {
+				nodes[0] = make_uint4(opt_info(T_LITERAL, 1, ctx), 0, rep0, rep1);
+				nodes[1] = make_uint4(rep2, rep3, 0, 0);
+			}
+			__syncwarp();
+			for (uint32_t j = 0; j < B; j++) {
+				const uint4 na = nodes[2 * j], nb = nodes[2 * j + 1];
+				const uint32_t c0 = s.cost[j], uctx = na.x >> 24;
+				const uint32_t rep[4] = {na.z, na.w, nb.x, nb.y};
+				const uint32_t i = p + j, maxl = B - j < 273 ? B - j : 273;
+				// how far each rep distance matches (0 = not legal here), 32 bytes per step
+				uint32_t rl[4];
+				for (int q = 0; q < 4; q++) {
+					rl[q] = 0;
+					if (rep[q] < i) {
+						rl[q] = maxl;
+						for (uint32_t base = 0; base < maxl; base += 32) {
+							const uint32_t k = base + lane;
+							const bool differ = k < maxl && a.data[i + k] != a.data[i + k - rep[q] - 1];
+							const uint32_t bal = __ballot_sync(FULL, differ);
+							if (bal) {
+								rl[q] = base + __ffs(bal) - 1;
+								break;
+							}
+						}
+					}
+				}
+				// the match list: entry e's distance price for each length context, in shared memory
+				const uint32_t count = a.counts[i];
+				if (lane < count) {
+					const uint2 en = a.lists[(size_t)i * OPT_LIST + lane];
+					s.ent_len[lane] = en.x;
+					s.ent_dist[lane] = en.y;
+					const uint32_t dist = en.y;
+					uint32_t extra = 0, pslot = dist;
+					if (dist >= 4) {
+						const uint32_t nlow = 30u - (uint32_t)__clz(dist), low = dist & ((1u << nlow) - 1), high = dist >> nlow;
+						pslot = nlow * 2 + high;
+						extra = pslot < 14 ? opt_tree_rev(s, DS_POSCODER + (high << nlow) - pslot, nlow, low)
+						                   : ((nlow - 4) << 11) + s.alignp[low & 15];
+					}
+					for (int c = 0; c < 4; c++) s.ent_dp[lane][c] = s.slotp[c][pslot] + extra;
+				}
+				__syncwarp();
+				const uint32_t is_rep = opt_bit(s, DS_ISMATCH + (uctx << 4), 1) + opt_bit(s, DS_ISREP + uctx, 1);
+				uint32_t rep_head[4];
+				rep_head[0] = is_rep + opt_bit(s, DS_ISREPG0 + uctx, 0) + opt_bit(s, DS_ISREP0LONG + (uctx << 4), 1);
+				const uint32_t g0 = is_rep + opt_bit(s, DS_ISREPG0 + uctx, 1);
+				rep_head[1] = g0 + opt_bit(s, DS_ISREPG1 + uctx, 0);
+				rep_head[2] = g0 + opt_bit(s, DS_ISREPG1 + uctx, 1) + opt_bit(s, DS_ISREPG2 + uctx, 0);
+				rep_head[3] = g0 + opt_bit(s, DS_ISREPG1 + uctx, 1) + opt_bit(s, DS_ISREPG2 + uctx, 1);
+				const uint32_t match_head = opt_bit(s, DS_ISMATCH + (uctx << 4), 1) + opt_bit(s, DS_ISREP + uctx, 0);
+				uint32_t e = 0;
+				for (uint32_t l = lane; l <= maxl; l += 32) {
+					if (l == 0) continue;
+					uint32_t best = OPT_INF, type = 0, dist = 0;
+					if (l == 1) {
+						// LITERAL (matched against rep0 after a match or rep), then SHORT_REP
+						const uint32_t byte = a.data[i];
+						best = opt_bit(s, DS_ISMATCH + (uctx << 4), 0);
+						if (uctx < 7) {
+							best += s.litp[byte];
+						} else {
+							const uint32_t mbyte = a.data[i - rep[0] - 1];
+							bool matched = true;
+							uint32_t node = 1;
+							for (int b = 7; b >= 0; b--) {
+								const uint32_t bit = (byte >> b) & 1u;
+								uint32_t slot = node;
+								if (matched) {
+									const uint32_t mbit = (mbyte >> b) & 1u;
+									slot += (1u + mbit) << 8;
+									matched = mbit == bit;
+								}
+								best += opt_bit(s, DS_LIT + slot, bit);
+								node = (node << 1) | bit;
+							}
+						}
+						type = T_LITERAL;
+						if (rep[0] < i && byte == a.data[i - rep[0] - 1]) {
+							const uint32_t c = is_rep + opt_bit(s, DS_ISREPG0 + uctx, 0) + opt_bit(s, DS_ISREP0LONG + (uctx << 4), 0);
+							if (c < best) {
+								best = c;
+								type = T_SHORT_REP;
+							}
+						}
+					} else {
+						for (int q = 0; q < 4; q++) {
+							if (rl[q] < l) continue;
+							const uint32_t c = rep_head[q] + s.lenp[1][l];
+							if (c < best) {
+								best = c;
+								type = T_LONG_REP;
+								dist = (uint32_t)q;
+							}
+						}
+						while (e < count && s.ent_len[e] < l) e++;
+						if (e < count) {
+							const uint32_t c = match_head + s.lenp[0][l] + s.ent_dp[e][l - 2 < 3 ? l - 2 : 3];
+							if (c < best) {
+								best = c;
+								type = T_MATCH;
+								dist = s.ent_dist[e];
+							}
+						}
+					}
+					if (best == OPT_INF || c0 + best >= s.cost[j + l]) continue;
+					s.cost[j + l] = c0 + best;
+					// the target's state: src/lzma_state.c:29-81
+					uint32_t r0 = rep[0], r1 = rep[1], r2 = rep[2], r3 = rep[3];
+					if (type == T_MATCH) {
+						r3 = r2;
+						r2 = r1;
+						r1 = r0;
+						r0 = dist;
+					} else if (type == T_LONG_REP) {
+						const uint32_t d = rep[dist];
+						if (dist > 2) r3 = r2;
+						if (dist > 1) r2 = r1;
+						if (dist > 0) r1 = r0;
+						r0 = d;
+					}
+					nodes[2 * (j + l)] = make_uint4(opt_info(type, l, next_ctx(uctx, type)), dist, r0, r1);
+					nodes[2 * (j + l) + 1] = make_uint4(r2, r3, 0, 0);
+				}
+				__syncwarp();
+			}
+			// commit: mark the cheapest path in the slab, then run the exact model through it
+			if (lane == 0) {
+				for (uint32_t j = B; j > 0;) {
+					const uint4 na = nodes[2 * j];
+					const uint32_t type = na.x & 0xffu, len = (na.x >> 8) & 0xffffu;
+					j -= len;
+					a.slab[p + j] = pk_pack(type, na.y, len);
+				}
+				for (uint32_t q = p; q < p + B;) {
+					const uint64_t pk = a.slab[q];
+					const uint32_t type = pk_type(pk), len = pk_len(pk), dist = pk_dist(pk);
+					opt_code_packet(s, a.data, q, ctx, rep0, type, len, dist);
+					if (type == T_MATCH) {
+						rep3 = rep2;
+						rep2 = rep1;
+						rep1 = rep0;
+						rep0 = dist;
+					} else if (type == T_LONG_REP) {
+						const uint32_t d = dist == 0 ? rep0 : dist == 1 ? rep1 : dist == 2 ? rep2 : rep3;
+						a.abs_dist[q] = d + 1u;  // what the packet stands for, for the seam repair
+						if (dist > 2) rep3 = rep2;
+						if (dist > 1) rep2 = rep1;
+						if (dist > 0) rep1 = rep0;
+						rep0 = d;
+					}
+					ctx = next_ctx(ctx, type);
+					q += len;
+				}
+			}
+			ctx = __shfl_sync(FULL, ctx, 0);
+			rep0 = __shfl_sync(FULL, rep0, 0);
+			rep1 = __shfl_sync(FULL, rep1, 0);
+			rep2 = __shfl_sync(FULL, rep2, 0);
+			rep3 = __shfl_sync(FULL, rep3, 0);
+			relaxed += B;
+			p += B;
+		}
+	}
+	if (lane == 0 && relaxed) atomicAdd(a.nodes_relaxed, relaxed);
+}
+
 }  // namespace mg

@@ -19,6 +19,9 @@
  * --resume FILE starts the search from the slab of an .lzma stream of the same input (an earlier output, or
  * liblzma's with lc = lp = pb = 0), decoded on the device by mg_decode_stream, instead of from zero; the run
  * never writes a slab costlier than the one it read.
+ *
+ * --optimal N starts the rounds from a shortest-path parse of N regions built on the device
+ * (mg_anneal_optimal_init) instead of from the all-literal slab.
  */
 #include <pthread.h>
 #include <stdio.h>
@@ -34,12 +37,12 @@ static void usage(const char* argv0)
 	fprintf(stderr,
 	        "usage: %s [--chains N] [--iters N] [--epochs N] [--steps N] [--seed N] [--device N] [--gpus N] [--top-k N]\n"
 	        "          [--rounds N | --time SECONDS] [--round-ms N] [--group N] [--temp T] [--sm-khz N]\n"
-	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS | --resume FILE] filename\n",
+	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS | --optimal REGIONS | --resume FILE] filename\n",
 	        argv0);
 }
 
 typedef struct {
-	unsigned chains, iters, epochs, steps, device, top_k, rounds, round_ms, group, temp0, gpus, sm_khz, window, max_occ, greedy;
+	unsigned chains, iters, epochs, steps, device, top_k, rounds, round_ms, group, temp0, gpus, sm_khz, window, max_occ, greedy, optimal;
 	unsigned long long seed;
 	const uint8_t* data;
 	size_t size;
@@ -121,6 +124,14 @@ static int run_rounds(Worker* w, mg_anneal* an)
 		uint64_t cost = 0;
 		if (mg_anneal_greedy_init(an, c->greedy, 0, &cost)) return die(w, "mg_anneal_greedy_init");
 		if (mg_anneal_broadcast_chain(an, 0)) return die(w, "mg_anneal_broadcast_chain");
+	}
+	if (c->optimal) {
+		/* --optimal N: the same from a shortest-path parse of N regions (match lists of the default 64
+		 * occurrences; --max-occ limits the annealer's finder only) */
+		uint64_t cost = 0;
+		if (mg_anneal_optimal_init(an, c->optimal, 0, 0, &cost)) return die(w, "mg_anneal_optimal_init");
+		if (mg_anneal_broadcast_chain(an, 0)) return die(w, "mg_anneal_broadcast_chain");
+		if (w->rank == 0) fprintf(stderr, "current file size: %f\toptimal parse (%u regions)\n", 18 + cost / 16384.f, c->optimal);
 	}
 	unsigned long long lcg = c->seed, evals = 0;
 	double device_ms = 0;
@@ -395,6 +406,7 @@ int main(int argc, char** argv)
 		else if (!strcmp(a, "--window")) target = &cfg.window;   /* match-finder limits for huge inputs; 0 = the */
 		else if (!strcmp(a, "--max-occ")) target = &cfg.max_occ; /* reference's unbounded enumeration */
 		else if (!strcmp(a, "--greedy")) target = &cfg.greedy;   /* start the rounds from a greedy parse of N regions */
+		else if (!strcmp(a, "--optimal")) target = &cfg.optimal; /* ... or from a shortest-path parse of N regions */
 		if (target) {
 			if (++i >= argc) { usage(argv[0]); return -1; }
 			*target = (unsigned)strtoul(argv[i], NULL, 10);
@@ -416,7 +428,8 @@ int main(int argc, char** argv)
 	}
 	if (time_s > 0 && cfg.round_ms > 0) cfg.rounds = (time_s * 1000u + cfg.round_ms - 1) / cfg.round_ms;
 	if (filename == NULL || cfg.chains == 0 || cfg.gpus == 0 || cfg.gpus > 64 ||
-	    (cfg.rounds == 0 && (cfg.steps == 0 || cfg.epochs == 0)) || (resume_name && cfg.greedy)) {
+	    (cfg.rounds == 0 && (cfg.steps == 0 || cfg.epochs == 0)) || (resume_name && cfg.greedy) ||
+	    (cfg.optimal && (cfg.greedy || resume_name || cfg.rounds == 0))) {
 		usage(argv[0]);
 		return -1;
 	}
