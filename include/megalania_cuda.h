@@ -144,6 +144,28 @@ MG_API int mg_encode_slab_buffer(mg_ctx* ctx, const LZMAPacket* slab, uint8_t* o
  * by the last mg_encode_slab / mg_encode_slab_buffer on ctx. */
 MG_API int mg_encode_stats(const mg_ctx* ctx, double* kernel_ms, uint64_t* events);
 
+/* ---- .xz output ------------------------------------------------------------------------- */
+
+/* The same slab as one .xz stream (no reference counterpart: the reference writes LZMA-alone only): one block, the
+ * CRC64 check, LZMA2 at lc = lp = pb = 0 with a dictionary of at least max(n, 4 KiB).  The first LZMA2 chunk resets
+ * the dictionary and state and sets the properties; every later chunk resets nothing - it keeps the probabilities,
+ * automaton state and rep distances of the chunk before it - and restarts only the range coder.  So every chunk is
+ * range-coded on its own, all of them side by side on the device, and the stream prices exactly as the .lzma one
+ * plus about 60 bytes of container and 5 per chunk header.
+ *   Cut candidates: the first packet boundary at or after each multiple of 4096 below n, and n; the cost of
+ *   everything before a candidate comes from one pricing walk of the slab (the cost of mg_score_slabs).
+ *   Chunk plan: a chunk starts at 0 or at the previous chunk's end s, and ends at the farthest candidate e > s whose
+ *   priced cost(s, e) is at most chunk_bytes * 8 bits (chunk_bytes * 8 * 2048 in the units of mg_score_slabs) with
+ *   e - s <= 2 MiB; when no candidate qualifies, at the nearest candidate after s.
+ * chunk_bytes: 0 = 61440 (liblzma's own chunk target), else 256..61440.  A chunk's coded size never exceeds the
+ * 65536 bytes an LZMA2 chunk holds (DESIGN.md §4 K8); a chunk that did would fail the call with MG_ESLAB naming the
+ * chunk, and nothing would be written.  The stream is handed to `out` in one write.
+ *   MG_EINVAL: chunk_bytes out of range.  MG_ESLAB: an undecodable slab, as for mg_encode_slab. */
+MG_API int mg_encode_slab_xz(mg_ctx* ctx, const LZMAPacket* slab, uint32_t chunk_bytes, OutputInterface* out);
+/* Device time (CUDA events) of the last mg_encode_slab_xz's plan walk and of its chunk kernel, its chunk count and
+ * the events its chunks coded (the unit of mg_encode_stats: the same slab codes the same events either way). */
+MG_API int mg_encode_xz_stats(const mg_ctx* ctx, double* plan_ms, double* code_ms, uint32_t* chunks, uint64_t* events);
+
 /* ---- stream -> slab: resume from an existing .lzma stream --------------------------------- */
 
 /* Replaces nothing in the reference (it has no way to read its output back).  Decodes an LZMA-alone stream of the

@@ -5,6 +5,7 @@ The names follow the reference's vocabulary (slab, packet, top-k finder, perplex
   Context.score_slabs(slabs)    perplexity_encoder total of a slab          (src/perplexity_encoder.c)
   Context.find_topk(...)        top_k_packet_finder_find + pop loop         (src/top_k_packet_finder.c)
   Context.encode_slab(slab)     header + range_encoder pass                 (src/main.c:110-119)
+  Context.encode_xz(slab)       the same slab as an .xz stream, LZMA2 chunks coded side by side  (no reference counterpart)
   Context.decode_stream(stream) .lzma stream (lc = lp = pb = 0) -> slab, to resume a search (no reference counterpart)
   Annealer.optimal_init(...)    shortest-path parse as a starting slab                           (no reference counterpart)
   Annealer(ctx, chains, ...)    the loop of src/main.c:78-102 on many chains
@@ -89,7 +90,8 @@ EXPORTS = [
     "mg_comm_unique_id", "mg_comm_init", "mg_comm_destroy", "mg_comm_rank", "mg_comm_size", "mg_comm_exchange_best",
     "mg_comm_temper_exchange", "mg_temper_decide", "mg_comm_merge_regions", "mg_comm_stats", "mg_pool_trim",
     "mg_comm_broadcast_chain", "mg_comm_allgather_u64", "mg_ctx_set_finder_limits", "mg_anneal_greedy_init",
-    "mg_decode_stream", "mg_decode_stats", "mg_anneal_optimal_init", "mg_optimal_stats",
+    "mg_decode_stream", "mg_decode_stats", "mg_anneal_optimal_init", "mg_optimal_stats", "mg_encode_slab_xz",
+    "mg_encode_xz_stats",
 ]
 
 _lib = None
@@ -173,6 +175,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.mg_decode_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
     L.mg_anneal_optimal_init.argtypes = [vp, u32, u32, u32, C.POINTER(u64)]
     L.mg_optimal_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(u64)]
+    L.mg_encode_slab_xz.argtypes = [vp, vp, u32, C.POINTER(OutputInterface)]
+    L.mg_encode_xz_stats.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(u32), C.POINTER(u64)]
     _lib = L
     return L
 
@@ -293,6 +297,25 @@ class Context:
         _check(self._lib.mg_encode_slab_buffer(self._h, _slab_ptr(slab, self.n), out.ctypes.data_as(C.c_void_p), cap,
                                                C.byref(got)))
         return out[:got.value].tobytes()
+
+    def encode_xz(self, slab: np.ndarray, chunk_bytes: int = 0) -> bytes:
+        """mg_encode_slab_xz: the slab as one .xz stream (one block, CRC64, LZMA2 chunks of at most chunk_bytes priced
+        bytes, 0 = 61440, else 256..61440)."""
+        chunks: list[bytes] = []
+
+        def _write(_iface, ptr, size):
+            chunks.append(C.string_at(ptr, size))
+            return True
+
+        iface = OutputInterface(WRITE_FN(_write), None)
+        _check(self._lib.mg_encode_slab_xz(self._h, _slab_ptr(as_slab(slab), self.n), chunk_bytes, C.byref(iface)))
+        return b"".join(chunks)
+
+    def encode_xz_stats(self) -> dict:
+        """Device time of the last encode_xz's plan walk and chunk kernel, its chunk count and coded events."""
+        plan, code, chunks, ev = C.c_double(0), C.c_double(0), C.c_uint32(0), C.c_uint64(0)
+        _check(self._lib.mg_encode_xz_stats(self._h, C.byref(plan), C.byref(code), C.byref(chunks), C.byref(ev)))
+        return {"plan_ms": plan.value, "code_ms": code.value, "chunks": int(chunks.value), "events": int(ev.value)}
 
     def decode_stream(self, stream: bytes) -> np.ndarray:
         """An LZMA-alone stream of this input (lc = lp = pb = 0: an earlier output, or liblzma's) -> the slab that

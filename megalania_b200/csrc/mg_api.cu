@@ -122,7 +122,7 @@ extern "C" MG_API void mg_pool_trim(void)
 	cudaSetDevice(device);
 }
 
-extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 3u; }
+extern "C" MG_API uint32_t mg_version(void) { return (0u << 16) | 4u; }
 
 struct mg_comm_state;
 
@@ -150,6 +150,10 @@ struct mg_ctx {
 	unsigned long long last_decode_events = 0;
 	double last_optimal_ms = 0;       // mg_anneal_optimal_init: device time and nodes of the last call
 	unsigned long long last_optimal_nodes = 0;
+	double last_xz_plan_ms = 0;       // mg_encode_slab_xz: device time of the plan walk and of the chunk kernel,
+	double last_xz_code_ms = 0;       // chunks and events of the last call
+	uint32_t last_xz_chunks = 0;
+	unsigned long long last_xz_events = 0;
 };
 
 struct DevBuf {
@@ -180,6 +184,7 @@ static int set_smem_attrs()
 	CU(cudaFuncSetAttribute(anneal_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CtaShared)));
 	CU(cudaFuncSetAttribute(greedy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CtaShared)));
 	CU(cudaFuncSetAttribute(encode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(EncodeShared)));
+	CU(cudaFuncSetAttribute(encode_chunks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CHUNK_SMEM));
 	// the model lives in shared memory: ask for the largest carve-out so that occupancy is set by registers
 	CU(cudaFuncSetAttribute(score_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
 	CU(cudaFuncSetAttribute(topk_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -746,6 +751,267 @@ extern "C" MG_API int mg_encode_slab_buffer(mg_ctx* ctx, const LZMAPacket* slab,
 	if (*out_len > cap) return fail(MG_EINVAL, "mg_encode_slab_buffer: need %zu bytes, have %zu", *out_len, cap);
 	make_header(ctx, out);
 	memcpy(out + 13, payload.data(), payload.size());
+	return MG_OK;
+}
+
+// ---- .xz: LZMA2 chunks coded side by side ---------------------------------------------------------------------
+constexpr uint32_t XZ_GRANULE = 4096;          // the plan walk's checkpoint stride: cut candidates every 4 KiB
+constexpr uint32_t XZ_CHUNK_DEFAULT = 61440;   // liblzma's own target for an LZMA2 chunk's coded bytes
+constexpr uint32_t XZ_CHUNK_MIN = 256;
+constexpr uint32_t LZMA2_MAX_U = 1u << 21;     // an LZMA2 chunk holds at most 2 MiB of input ...
+constexpr uint32_t LZMA2_MAX_C = 1u << 16;     // ... and at most 64 KiB of coded bytes
+
+static uint32_t crc32_update(uint32_t crc, const uint8_t* p, size_t len)
+{
+	static uint32_t table[256];
+	static bool ready = false;
+	if (!ready) {
+		for (uint32_t i = 0; i < 256; i++) {
+			uint32_t c = i;
+			for (int k = 0; k < 8; k++) c = (c >> 1) ^ (0xEDB88320u & (0u - (c & 1u)));
+			table[i] = c;
+		}
+		ready = true;
+	}
+	crc = ~crc;
+	for (size_t i = 0; i < len; i++) crc = table[(crc ^ p[i]) & 0xff] ^ (crc >> 8);
+	return ~crc;
+}
+
+static uint64_t crc64_update(uint64_t crc, const uint8_t* p, size_t len)
+{
+	static uint64_t table[256];
+	static bool ready = false;
+	if (!ready) {
+		for (uint64_t i = 0; i < 256; i++) {
+			uint64_t c = i;
+			for (int k = 0; k < 8; k++) c = (c >> 1) ^ (0xC96C5795D7870F42ull & (0ull - (c & 1ull)));
+			table[i] = c;
+		}
+		ready = true;
+	}
+	crc = ~crc;
+	for (size_t i = 0; i < len; i++) crc = table[(crc ^ p[i]) & 0xff] ^ (crc >> 8);
+	return ~crc;
+}
+
+static void put_le(std::vector<uint8_t>& v, uint64_t x, int bytes)
+{
+	for (int i = 0; i < bytes; i++) v.push_back((uint8_t)(x >> (8 * i)));
+}
+
+static void put_varint(std::vector<uint8_t>& v, uint64_t x)
+{
+	while (x >= 0x80) {
+		v.push_back((uint8_t)(x | 0x80));
+		x >>= 7;
+	}
+	v.push_back((uint8_t)x);
+}
+
+static void pad4(std::vector<uint8_t>& v, size_t from)
+{
+	while ((v.size() - from) & 3) v.push_back(0);
+}
+
+// The smallest LZMA2 dictionary-size byte whose size, (2 | (b & 1)) << (b / 2 + 11), is at least max(n, 4 KiB).
+static uint8_t lzma2_dict_byte(uint32_t n)
+{
+	uint8_t b = 0;
+	while (b < 40 && ((uint64_t)(2u | (b & 1u)) << (b / 2 + 11)) < n) b++;
+	return b;
+}
+
+// One .xz stream: one block, LZMA2 (lc = lp = pb = 0), check CRC64.  chunk c holds the input [bounds[c],
+// bounds[c + 1]) range-coded in payload[c].
+static std::vector<uint8_t> xz_stream(const uint8_t* input, uint32_t n, const std::vector<uint32_t>& bounds,
+                                      const std::vector<std::vector<uint8_t>>& payload)
+{
+	std::vector<uint8_t> v;
+	const uint8_t magic[6] = {0xFD, '7', 'z', 'X', 'Z', 0x00}, flags[2] = {0x00, 0x04};  // flags: check = CRC64
+	v.insert(v.end(), magic, magic + 6);
+	v.insert(v.end(), flags, flags + 2);
+	put_le(v, crc32_update(0, flags, 2), 4);
+	// block header: size, flags (one filter, no size fields), LZMA2 with its dictionary byte, padding, CRC32
+	const size_t block = v.size();
+	v.push_back(0);
+	v.push_back(0x00);
+	v.push_back(0x21);
+	v.push_back(0x01);
+	v.push_back(lzma2_dict_byte(n));
+	pad4(v, block);
+	v[block] = (uint8_t)((v.size() + 4 - block) / 4 - 1);
+	put_le(v, crc32_update(0, v.data() + block, v.size() - block), 4);
+	// LZMA2 chunks: the first resets the dictionary and state and sets the properties (byte 0: lc = lp = pb = 0), the
+	// rest keep everything and restart only the range coder
+	for (size_t c = 0; c + 1 < bounds.size(); c++) {
+		const uint32_t u = bounds[c + 1] - bounds[c] - 1, z = (uint32_t)payload[c].size() - 1;
+		v.push_back((uint8_t)((c == 0 ? 0xE0u : 0x80u) | (u >> 16)));
+		v.push_back((uint8_t)(u >> 8));
+		v.push_back((uint8_t)u);
+		v.push_back((uint8_t)(z >> 8));
+		v.push_back((uint8_t)z);
+		if (c == 0) v.push_back(0x00);
+		v.insert(v.end(), payload[c].begin(), payload[c].end());
+	}
+	v.push_back(0x00);  // end of the LZMA2 data
+	const uint64_t unpadded = v.size() - block + 8;
+	pad4(v, block);
+	put_le(v, crc64_update(0, input, n), 8);
+	// index: one record (unpadded block size, input size), padding, CRC32
+	const size_t index = v.size();
+	v.push_back(0x00);
+	put_varint(v, 1);
+	put_varint(v, unpadded);
+	put_varint(v, n);
+	pad4(v, index);
+	put_le(v, crc32_update(0, v.data() + index, v.size() - index), 4);
+	const uint32_t backward = (uint32_t)((v.size() - index) / 4 - 1);
+	// stream footer: CRC32 of (backward size, flags), backward size, flags, "YZ"
+	uint8_t tail[6];
+	for (int i = 0; i < 4; i++) tail[i] = (uint8_t)(backward >> (8 * i));
+	tail[4] = flags[0];
+	tail[5] = flags[1];
+	put_le(v, crc32_update(0, tail, 6), 4);
+	v.insert(v.end(), tail, tail + 6);
+	v.push_back('Y');
+	v.push_back('Z');
+	return v;
+}
+
+extern "C" MG_API int mg_encode_slab_xz(mg_ctx* ctx, const LZMAPacket* slab, uint32_t chunk_bytes, OutputInterface* out)
+{
+	if (!ctx || !slab || !out || !out->write) return fail(MG_EINVAL, "mg_encode_slab_xz: null argument");
+	if (chunk_bytes == 0) chunk_bytes = XZ_CHUNK_DEFAULT;
+	if (chunk_bytes < XZ_CHUNK_MIN || chunk_bytes > XZ_CHUNK_DEFAULT)
+		return fail(MG_EINVAL, "mg_encode_slab_xz: chunk_bytes %u is outside %u..%u", chunk_bytes, XZ_CHUNK_MIN, XZ_CHUNK_DEFAULT);
+	CU(cudaSetDevice(ctx->device));
+	const uint32_t n = ctx->n;
+	// plan walk: one score_kernel pass with a checkpoint at the first packet boundary at or after each multiple of
+	// the granule (a packet is at most 273 bytes, so none is skipped; one that falls on n is not written)
+	const uint32_t nrec = (n - 1) / XZ_GRANULE;
+	DevBuf packed, ck, meta, cost, err;
+	if (int rc = dev_alloc(packed, (size_t)n * 8)) return rc;
+	if (int rc = dev_alloc(ck, (size_t)(nrec ? nrec : 1) * sizeof(Record))) return rc;
+	if (int rc = dev_alloc(meta, (size_t)(nrec ? nrec : 1) * sizeof(CkMeta))) return rc;
+	if (int rc = dev_alloc(cost, 8)) return rc;
+	if (int rc = dev_alloc(err, 4)) return rc;
+	if (int rc = upload_packed(ctx, slab, n, packed.as<uint64_t>())) return rc;
+	CU(cudaMemsetAsync(meta.p, 0xff, (size_t)(nrec ? nrec : 1) * sizeof(CkMeta), ctx->stream));
+	cudaEvent_t ev[4];
+	for (auto& e : ev) CU(cudaEventCreate(&e));
+	struct Events {
+		cudaEvent_t* e;
+		~Events() { for (int i = 0; i < 4; i++) cudaEventDestroy(e[i]); }
+	} events_guard{ev};
+	CU(cudaEventRecord(ev[0], ctx->stream));
+	if (int rc = score_device(ctx, packed.as<uint64_t>(), 1, n, cost.as<uint64_t>(), nullptr, err.as<uint32_t>(),
+	                          nrec ? ck.as<Record>() : nullptr, nullptr, meta.as<CkMeta>(), XZ_GRANULE, nrec + 1, nullptr))
+		return rc;
+	CU(cudaEventRecord(ev[1], ctx->stream));
+	std::vector<CkMeta> hmeta(nrec);
+	uint64_t total = 0;
+	uint32_t herr = 0;
+	if (nrec) CU(cudaMemcpyAsync(hmeta.data(), meta.p, nrec * sizeof(CkMeta), cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaMemcpyAsync(&total, cost.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaMemcpyAsync(&herr, err.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	if (herr) return fail(MG_ESLAB, "mg_encode_slab_xz: %s", walk_error(herr));
+	float plan_ms = 0;
+	cudaEventElapsedTime(&plan_ms, ev[0], ev[1]);
+
+	// cut candidates: the checkpoints and n, with the cost of everything before them
+	struct Cut {
+		uint32_t pos, rec;
+		uint64_t cost;
+	};
+	std::vector<Cut> cuts;
+	cuts.push_back({0, NO_RECORD, 0});
+	uint64_t acc = 0;
+	for (uint32_t i = 0; i < nrec && hmeta[i].pos != 0xffffffffu; i++) {
+		acc += hmeta[i].dcost;
+		cuts.push_back({hmeta[i].pos, i, acc});
+	}
+	cuts.push_back({n, NO_RECORD, total});
+	// chunk plan: from s, the farthest candidate e with cost(s, e) <= chunk_bytes * 8 bits and e - s <= 2 MiB, or the
+	// nearest one when none qualifies (costs only grow with e, so the qualifying candidates are the first ones)
+	const uint64_t budget = (uint64_t)chunk_bytes * 8 * 2048;
+	std::vector<uint32_t> bounds, start_rec;
+	for (size_t s = 0; s + 1 < cuts.size();) {
+		size_t e = s + 1;
+		while (e + 1 < cuts.size() && cuts[e + 1].cost - cuts[s].cost <= budget && cuts[e + 1].pos - cuts[s].pos <= LZMA2_MAX_U) e++;
+		bounds.push_back(cuts[s].pos);
+		start_rec.push_back(cuts[s].rec);
+		s = e;
+	}
+	bounds.push_back(n);
+	const uint32_t chunks = (uint32_t)start_rec.size();
+
+	// the chunks, one CTA each; a slot of 64 KiB per chunk (the coder counts what it could not store)
+	DevBuf dbounds, drec, dout, dres;
+	if (int rc = dev_alloc(dbounds, bounds.size() * 4)) return rc;
+	if (int rc = dev_alloc(drec, (size_t)chunks * 4)) return rc;
+	if (int rc = dev_alloc(dout, (size_t)chunks * LZMA2_MAX_C)) return rc;
+	if (int rc = dev_alloc(dres, (size_t)chunks * 12)) return rc;
+	CU(cudaMemcpyAsync(dbounds.p, bounds.data(), bounds.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+	CU(cudaMemcpyAsync(drec.p, start_rec.data(), (size_t)chunks * 4, cudaMemcpyHostToDevice, ctx->stream));
+	ChunkArgs a;
+	a.enc.data = ctx->d_data;
+	a.enc.n = n;
+	a.enc.slab = packed.as<uint64_t>();
+	a.enc.out = dout.as<uint8_t>();
+	a.enc.cap = LZMA2_MAX_C;
+	a.enc.out_len = dres.as<uint32_t>();
+	a.enc.out_err = dres.as<uint32_t>() + chunks;
+	a.enc.out_events = dres.as<uint32_t>() + 2 * (size_t)chunks;
+	a.enc.out_wait = nullptr;
+	a.enc.tables = ctx->tables;
+	a.ck = ck.as<Record>();
+	a.bounds = dbounds.as<uint32_t>();
+	a.start_rec = drec.as<uint32_t>();
+	CU(cudaEventRecord(ev[2], ctx->stream));
+	encode_chunks_kernel<<<chunks, 96, CHUNK_SMEM, ctx->stream>>>(a);
+	CU(cudaEventRecord(ev[3], ctx->stream));
+	CU(cudaGetLastError());
+	std::vector<uint32_t> res((size_t)chunks * 3);
+	CU(cudaMemcpyAsync(res.data(), dres.p, res.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	float code_ms = 0;
+	cudaEventElapsedTime(&code_ms, ev[2], ev[3]);
+	unsigned long long events = 0;
+	for (uint32_t c = 0; c < chunks; c++) events += res[2 * (size_t)chunks + c];
+	ctx->last_xz_plan_ms = plan_ms;
+	ctx->last_xz_code_ms = code_ms;
+	ctx->last_xz_chunks = chunks;
+	ctx->last_xz_events = events;
+	for (uint32_t c = 0; c < chunks; c++) {
+		const uint32_t len = res[c], e = res[(size_t)chunks + c];
+		if (e & ERR_BAD_PACKET) return fail(MG_ESLAB, "mg_encode_slab_xz: chunk %u: %s", c, walk_error(e));
+		if (len > LZMA2_MAX_C || e)
+			return fail(MG_ESLAB, "mg_encode_slab_xz: chunk %u (bytes %u..%u) codes to %u bytes, more than the %u an LZMA2 chunk holds",
+			            c, bounds[c], bounds[c + 1], len, LZMA2_MAX_C);
+	}
+	std::vector<std::vector<uint8_t>> payload(chunks);
+	for (uint32_t c = 0; c < chunks; c++) {
+		payload[c].resize(res[c]);
+		CU(cudaMemcpyAsync(payload[c].data(), dout.as<uint8_t>() + (size_t)c * LZMA2_MAX_C, res[c], cudaMemcpyDeviceToHost, ctx->stream));
+	}
+	// the block's check is the CRC64 of the input; the context keeps it on the device only
+	std::vector<uint8_t> input(n);
+	CU(cudaMemcpyAsync(input.data(), ctx->d_data, n, cudaMemcpyDeviceToHost, ctx->stream));
+	CU(cudaStreamSynchronize(ctx->stream));
+	const std::vector<uint8_t> stream = xz_stream(input.data(), n, bounds, payload);
+	if (!out->write(out, stream.data(), stream.size())) return fail(MG_EOUTPUT, "mg_encode_slab_xz: OutputInterface.write failed");
+	return MG_OK;
+}
+
+extern "C" MG_API int mg_encode_xz_stats(const mg_ctx* ctx, double* plan_ms, double* code_ms, uint32_t* chunks, uint64_t* events)
+{
+	if (!ctx) return fail(MG_EINVAL, "mg_encode_xz_stats: null context");
+	if (plan_ms) *plan_ms = ctx->last_xz_plan_ms;
+	if (code_ms) *code_ms = ctx->last_xz_code_ms;
+	if (chunks) *chunks = ctx->last_xz_chunks;
+	if (events) *events = ctx->last_xz_events;
 	return MG_OK;
 }
 

@@ -1652,11 +1652,26 @@ __device__ __forceinline__ uint32_t enc_event(uint32_t p, uint32_t bit) { return
 // The producer publishes `head` (a fence + a store) once per ENC_PUBLISH events, not per packet.
 constexpr uint32_t ENC_PUBLISH = 256;
 
-__device__ __forceinline__ void encode_produce(EncodeShared* sh, const EncodeArgs& a, int lane)
+// The packets of [m.pos, end): encode_kernel from a fresh model (start = null) up to n, encode_chunks_kernel from the
+// checkpoint record `start`, TMA-loaded on `bar`.  (The extra block and the copy of `end` keep encode_kernel's
+// machine code what it was before the chunk kernel shared this function.)
+__device__ __forceinline__ void encode_produce(EncodeShared* sh, const EncodeArgs& a, int lane, const Record* start,
+                                               uint32_t end, uint64_t* bar)
 {
 	Model m;
 	const SmemU16 probs{smem_u32(sh->rec.probs)};
-	model_init(lane, probs, m, 1024);  // the range coder keeps plain probabilities
+	{
+		if (start) {
+			uint64_t cost;
+			uint32_t parity = 0;
+			record_load(lane, &sh->rec, m, cost, start, bar, parity);
+			// the walk stores probabilities pre-shifted (p << PROB_SHIFT), the range coder keeps plain ones
+			for (uint32_t i = (uint32_t)lane; i < S_COUNT; i += 32) probs.set(i, probs.get(i) >> PROB_SHIFT);
+			__syncwarp();
+		} else {
+			model_init(lane, probs, m, 1024);
+		}
+	}
 	Window w;
 	w.base = WINDOW_NONE;
 	w.pf_base = WINDOW_NONE;
@@ -1676,7 +1691,8 @@ __device__ __forceinline__ void encode_produce(EncodeShared* sh, const EncodeArg
 	else if (tree && depth == 6) { lit_first = 2u * (S_LIT0 + 160); lit_sh = 1; lit_mask = 0x7e; lit_x = LITX6 << 1; lit_hm = 64; }
 	else if (tree && depth == 7) { lit_first = 2u * (S_LIT0 + 288); lit_sh = 0; lit_mask = 0xfe; lit_x = LITX7 << 1; lit_hm = 0xc0; }
 	const uint32_t lit_addr = probs.a + lit_first;
-	while (m.pos < a.n) {
+	const uint32_t stop = end;
+	while (m.pos < stop) {
 		// room for a whole window of literals (32 x 9 events; the largest other packet appends 28)?
 		if (head + 288 - tail_seen > ENC_RING) {
 			const long long t0 = clock64();
@@ -1699,7 +1715,7 @@ __device__ __forceinline__ void encode_produce(EncodeShared* sh, const EncodeArg
 			const uint32_t idx = m.pos - w.base;
 			uint32_t run = (uint32_t)__ffs((int)~(w.litmask >> idx)) - 1u;  // 0xffffffff when every slot up to the window's end is one
 			run = run < 32u - idx ? run : 32u - idx;
-			run = run < a.n - m.pos ? run : a.n - m.pos;
+			run = run < stop - m.pos ? run : stop - m.pos;
 			uint32_t cj = m.ctx;
 			uint32_t at = head + (uint32_t)lane;
 			for (uint32_t i = 0; i < run; i++) {
@@ -2006,11 +2022,54 @@ __global__ void __launch_bounds__(96) encode_kernel(EncodeArgs a)
 	}
 	__syncthreads();
 	if (threadIdx.x < 32)
-		encode_produce(&sh, a, (int)threadIdx.x);
+		encode_produce(&sh, a, (int)threadIdx.x, nullptr, a.n, nullptr);
 	else if (threadIdx.x == 32)
 		encode_range(&sh, a);
 	else if (threadIdx.x >= 64)
 		encode_low(&sh, a, (int)threadIdx.x - 64);
+}
+
+// ---- K8: the chunks of an LZMA2 stream, one CTA each ------------------------------------------------------
+// An LZMA2 chunk that resets nothing keeps the probabilities, automaton state and rep distances of the chunk before
+// it and restarts only the range coder.  So once the model at each chunk's start is known - a checkpoint record of
+// the plan walk (score_kernel) - every chunk is an independent LZMA-alone payload: encode_kernel's three strands
+// over [bounds[c], bounds[c + 1]), started from that record, with a fresh coder that flushes at the chunk's end.
+constexpr uint32_t NO_RECORD = 0xffffffffu;
+struct ChunkArgs {
+	EncodeArgs enc;             // data, n, slab; out = [chunks][enc.cap] bytes; out_len, out_err, out_events = [chunks]
+	const Record* ck;           // the plan walk's checkpoint records
+	const uint32_t* bounds;     // [chunks + 1]: chunk c codes [bounds[c], bounds[c + 1]), all packet boundaries
+	const uint32_t* start_rec;  // [chunks]: the record holding the model at bounds[c], NO_RECORD = a fresh model
+};
+constexpr size_t CHUNK_BAR_OFFSET = (sizeof(EncodeShared) + 7) & ~(size_t)7;
+constexpr size_t CHUNK_SMEM = CHUNK_BAR_OFFSET + sizeof(uint64_t);
+
+__global__ void __launch_bounds__(96) encode_chunks_kernel(ChunkArgs c)
+{
+	extern __shared__ __align__(128) unsigned char smem_raw[];
+	EncodeShared& sh = *reinterpret_cast<EncodeShared*>(smem_raw);
+	uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + CHUNK_BAR_OFFSET);
+	const uint32_t chunk = blockIdx.x;
+	EncodeArgs a = c.enc;
+	a.out += (size_t)chunk * a.cap;
+	a.out_len += chunk;
+	a.out_err += chunk;
+	a.out_events += chunk;
+	a.out_wait = nullptr;
+	if (threadIdx.x == 0) {
+		sh.head = sh.tail = sh.head_b = sh.tail_b = sh.done = sh.done_b = sh.err = 0;
+		mbar_init(bar, 1);
+		asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+	}
+	__syncthreads();
+	if (threadIdx.x < 32) {
+		const uint32_t r = c.start_rec[chunk];
+		encode_produce(&sh, a, (int)threadIdx.x, r == NO_RECORD ? nullptr : c.ck + r, c.bounds[chunk + 1], bar);
+	} else if (threadIdx.x == 32) {
+		encode_range(&sh, a);
+	} else if (threadIdx.x >= 64) {
+		encode_low(&sh, a, (int)threadIdx.x - 64);
+	}
 }
 
 // ---- slab format conversion: host LZMAPacket (12 B) <-> packed u64 ----------------------------------

@@ -22,6 +22,9 @@
  *
  * --optimal N starts the rounds from a shortest-path parse of N regions built on the device
  * (mg_anneal_optimal_init) instead of from the all-literal slab.
+ *
+ * --format xz writes the winning slab as an .xz stream (mg_encode_slab_xz: LZMA2 chunks range-coded side by side on
+ * the device) instead of .lzma; only the final write changes.
  */
 #include <pthread.h>
 #include <stdio.h>
@@ -37,7 +40,8 @@ static void usage(const char* argv0)
 	fprintf(stderr,
 	        "usage: %s [--chains N] [--iters N] [--epochs N] [--steps N] [--seed N] [--device N] [--gpus N] [--top-k N]\n"
 	        "          [--rounds N | --time SECONDS] [--round-ms N] [--group N] [--temp T] [--sm-khz N]\n"
-	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS | --optimal REGIONS | --resume FILE] filename\n",
+	        "          [--window BYTES] [--max-occ N] [--greedy REGIONS | --optimal REGIONS | --resume FILE]\n"
+	        "          [--format lzma|xz] filename\n",
 	        argv0);
 }
 
@@ -387,6 +391,7 @@ int main(int argc, char** argv)
 	unsigned time_s = 0; /* --time: annealing budget in seconds of SM time */
 	const char* filename = NULL;
 	const char* resume_name = NULL;
+	int xz = 0; /* --format: lzma (the reference's, the default) or xz */
 	for (int i = 1; i < argc; i++) {
 		const char* a = argv[i];
 		unsigned* target = NULL;
@@ -416,6 +421,9 @@ int main(int argc, char** argv)
 		} else if (!strcmp(a, "--resume")) {
 			if (++i >= argc) { usage(argv[0]); return -1; }
 			resume_name = argv[i];
+		} else if (!strcmp(a, "--format")) {
+			if (++i >= argc || (strcmp(argv[i], "lzma") && strcmp(argv[i], "xz"))) { usage(argv[0]); return -1; }
+			xz = !strcmp(argv[i], "xz");
 		} else if (a[0] == '-' && a[1] == '-') {
 			usage(argv[0]);
 			return -1;
@@ -503,8 +511,8 @@ int main(int argc, char** argv)
 	OutputInterface output;
 	StreamSink sink;
 	stream_sink_init(&output, &sink, stream_out);
-	if (mg_encode_slab(win->ctx, win->packets_best, &output)) {
-		fprintf(stderr, "mg_encode_slab: %s\n", mg_last_error());
+	if (xz ? mg_encode_slab_xz(win->ctx, win->packets_best, 0, &output) : mg_encode_slab(win->ctx, win->packets_best, &output)) {
+		fprintf(stderr, "%s: %s\n", xz ? "mg_encode_slab_xz" : "mg_encode_slab", mg_last_error());
 		return -1;
 	}
 	if (fflush(stream_out) != 0 || sink.failed) {
